@@ -49,6 +49,7 @@ typedef struct {
     uint8_t *pinned;            /* [N] */
     int32_t *sa, *sb;           /* spring endpoints, ptA (earlier point) / ptB (creating point) */
     uint8_t *stype;             /* 0 structural, 1 shearing, 2 bending */
+    uint8_t *skind;             /* creation kind k = 0..5 of cloth.pyx:135-146 (ptA = ptB - {W,1,W+1,W-1,2W,2}[k]) */
     double *rest;               /* [S] */
     int32_t *grabbed;           /* gripper.grabbed_pts, multiplicity preserved */
     int n_grabbed, cap_grabbed;
@@ -58,6 +59,11 @@ typedef struct {
     int32_t *map_next, *map_head, *map_tail;
     int64_t *map_key;
     int map_cap;
+    /* graph-coloured mode (oracle_update_coloured): not part of the reference */
+    int mode, relax_iters;
+    int32_t *corder;            /* spring indices by colour class, creation order within a class */
+    int32_t cstart[13];         /* class j = corder[cstart[j] .. cstart[j+1]) */
+    double *snap;               /* [N][3] post-Verlet snapshot of the Jacobi collision */
     /* instrumentation (not part of the reference): counters for design studies */
     int64_t n_updates, n_pair_tests, n_collide_hits, n_stretched, n_plane;
     int32_t *rec; int rec_cap, rec_n;   /* optional: indices of the springs shortened by the last limit pass */
@@ -86,10 +92,19 @@ int oracle_sizeof_params(void) { return (int)sizeof(OracleParams); }
 void oracle_cloth_destroy(OracleCloth *c) {
     if (!c) return;
     free(c->pos); free(c->prev); free(c->force); free(c->pinned);
-    free(c->sa); free(c->sb); free(c->stype); free(c->rest); free(c->grabbed);
+    free(c->sa); free(c->sb); free(c->stype); free(c->skind); free(c->rest); free(c->grabbed);
+    free(c->corder); free(c->snap);
     free(c->map_next); free(c->map_head); free(c->map_tail); free(c->map_key);
     free(c->rec);
     free(c);
+}
+
+/* Colour class 2k + parity of spring s, created by ptB = (r, c) with kind k: the parity is that of r for k = 0, 2, 3,
+ * of c for k = 1, of r >> 1 for k = 4 and of c >> 1 for k = 5.  Two springs of one class share no point. */
+static int spring_class(const OracleCloth *c, int s) {
+    int W = c->P.num_width_points, b = c->sb[s], r = b / W, cc = b % W, k = c->skind[s];
+    int key = (k == 1) ? cc : (k == 4 ? (r >> 1) : (k == 5 ? (cc >> 1) : r));
+    return 2 * k + (key & 1);
 }
 
 /* Cloth.__init__ grid + spring construction, cloth.pyx:92-146, Spring.__init__ :411-417.
@@ -111,6 +126,9 @@ OracleCloth *oracle_cloth_create(const OracleParams *P, int init_type, const dou
     c->sa = (int32_t *)malloc(6 * N * sizeof(int32_t));
     c->sb = (int32_t *)malloc(6 * N * sizeof(int32_t));
     c->stype = (uint8_t *)malloc(6 * N);
+    c->skind = (uint8_t *)malloc(6 * N);
+    c->corder = (int32_t *)malloc(6 * N * sizeof(int32_t));
+    c->snap = (double *)calloc(3 * N, sizeof(double));
     c->rest = (double *)malloc(6 * N * sizeof(double));
     c->cap_grabbed = 64;
     c->grabbed = (int32_t *)malloc(c->cap_grabbed * sizeof(int32_t));
@@ -138,24 +156,32 @@ OracleCloth *oracle_cloth_create(const OracleParams *P, int init_type, const dou
             }
             c->pos[3 * p] = x; c->pos[3 * p + 1] = y; c->pos[3 * p + 2] = z;
             c->prev[3 * p] = x; c->prev[3 * p + 1] = y; c->prev[3 * p + 2] = z; /* point.pyx:37-39 */
-#define ADD_SPRING(A, T)                                                              \
+#define ADD_SPRING(A, T, K)                                                           \
     do {                                                                              \
         int a_ = (A);                                                                 \
-        c->sa[S] = a_; c->sb[S] = p; c->stype[S] = (T);                               \
+        c->sa[S] = a_; c->sb[S] = p; c->stype[S] = (T); c->skind[S] = (K);            \
         c->rest[S] = fastnorm(c->pos[3 * a_] - x, c->pos[3 * a_ + 1] - y,             \
                               c->pos[3 * a_ + 2] - z); /* cloth.pyx:417 ptA - ptB */  \
         S++;                                                                          \
     } while (0)
-            if (r > 0) ADD_SPRING((r - 1) * W + cc, 0);                     /* :135-136 */
-            if (cc > 0) ADD_SPRING(r * W + cc - 1, 0);                      /* :137-138 */
-            if (r > 0 && cc > 0) ADD_SPRING((r - 1) * W + cc - 1, 1);       /* :139-140 */
-            if (r > 0 && cc + 1 < W) ADD_SPRING((r - 1) * W + cc + 1, 1);   /* :141-142 */
-            if (r > 1) ADD_SPRING((r - 2) * W + cc, 2);                     /* :143-144 */
-            if (cc > 1) ADD_SPRING(r * W + cc - 2, 2);                      /* :145-146 */
+            if (r > 0) ADD_SPRING((r - 1) * W + cc, 0, 0);                     /* :135-136 */
+            if (cc > 0) ADD_SPRING(r * W + cc - 1, 0, 1);                      /* :137-138 */
+            if (r > 0 && cc > 0) ADD_SPRING((r - 1) * W + cc - 1, 1, 2);       /* :139-140 */
+            if (r > 0 && cc + 1 < W) ADD_SPRING((r - 1) * W + cc + 1, 1, 3);   /* :141-142 */
+            if (r > 1) ADD_SPRING((r - 2) * W + cc, 2, 4);                     /* :143-144 */
+            if (cc > 1) ADD_SPRING(r * W + cc - 2, 2, 5);                      /* :145-146 */
 #undef ADD_SPRING
         }
     }
     c->S = S;
+    /* colour classes (DESIGN.md §4 "Coloured mode"): counting sort, stable in creation order */
+    memset(c->cstart, 0, sizeof(c->cstart));
+    for (int s = 0; s < S; s++) c->cstart[spring_class(c, s) + 1]++;
+    for (int j = 0; j < 12; j++) c->cstart[j + 1] += c->cstart[j];
+    int fill[12];
+    memcpy(fill, c->cstart, sizeof(fill));
+    for (int s = 0; s < S; s++) c->corder[fill[spring_class(c, s)]++] = s;
+    c->relax_iters = 1;
     return c;
 }
 
@@ -385,9 +411,108 @@ int oracle_update(OracleCloth *c) {
     return ORACLE_OK;
 }
 
+/* ---- Graph-coloured mode (CLOTHB200_MODE_COLOURED, DESIGN.md §4): the specification of the kernel's
+ * update_coloured(), NOT the reference's update.  The f64 coloured build equals it bit for bit: the Jacobi sums run
+ * in member-index order, and the springs of one colour class share no point, so running them in parallel equals
+ * running them in creation order.  Where the kernel's expression form was a free choice (squared compares, e*fac),
+ * that form is part of the definition. ---- */
+#define ORACLE_MODE_REFERENCE_ORDER 0
+#define ORACLE_MODE_COLOURED 1
+
+/* mode of every later update (oracle_update_n, oracle_run_plan); relax_iters limit passes, at least one */
+void oracle_cloth_set_mode(OracleCloth *c, int mode, int relax_iters) { c->mode = mode; c->relax_iters = relax_iters; }
+void oracle_cloth_get_colours(const OracleCloth *c, int32_t *out) {
+    for (int s = 0; s < c->S; s++) out[s] = spring_class(c, s);
+}
+
+/* Jacobi self-collision: every unpinned point is corrected from the post-Verlet snapshot of its bucket (members in
+ * index order, pinned members count); needs oracle_phase_build_map on the same positions. */
+int oracle_phase_self_collide_jacobi(OracleCloth *c) {
+    memcpy(c->snap, c->pos, 3 * c->N * sizeof(double));
+    double thresh = 2.0 * c->P.thickness;
+    int ss = c->P.simulation_steps;
+    for (int p = 0; p < c->N; p++) {
+        if (c->pinned[p]) continue;
+        const double *x = c->snap + 3 * p;
+        int64_t key;
+        int rc = hash_position(c, x[0], x[1], x[2], &key);
+        if (rc) return rc;
+        int slot = map_find_slot(c, key);
+        double t0 = 0.0, t1 = 0.0, t2 = 0.0;
+        int n = 0;
+        for (int q = c->map_head[slot]; q >= 0; q = c->map_next[q]) {
+            if (q == p) continue;
+            const double *y = c->snap + 3 * q;
+            double d = fastnorm(x[0] - y[0], x[1] - y[1], x[2] - y[2]);
+            c->n_pair_tests++;
+            if (d <= thresh) {
+                if (d == 0.0) return ORACLE_ERR_ZERODIV;
+                double factor = (thresh - d) / d;
+                t0 += (x[0] - y[0]) * factor;
+                t1 += (x[1] - y[1]) * factor;
+                t2 += (x[2] - y[2]) * factor;
+                n += 1;
+            }
+        }
+        if (n != 0) {
+            double nf = (double)n, *w = c->pos + 3 * p;
+            double c0 = t0 / nf / ss, c1 = t1 / nf / ss, c2 = t2 / nf / ss;
+            w[0] = w[0] + c0; w[1] = w[1] + c1; w[2] = w[2] + c2;
+            c->n_collide_hits += n;
+        }
+    }
+    return ORACLE_OK;
+}
+
+/* The 10 % limit in colour order: classes (k, parity) for k = 0..5, parity 0, 1; max(1, relax_iters) passes.
+ * Squared compares for the tear and the limit, correction e*fac with fac = (l - rest*1.1)/l. */
+void oracle_phase_limit_coloured(OracleCloth *c, int relax_iters) {
+    double tear_thresh = c->P.tear_thresh;
+    int passes = relax_iters > 1 ? relax_iters : 1;
+    c->rec_n = 0;
+    for (int it = 0; it < passes; it++) {
+        for (int j = 0; j < c->cstart[12]; j++) {
+            int s = c->corder[j], a = c->sa[s], b = c->sb[s];
+            int pa_ = c->pinned[a], pb_ = c->pinned[b];
+            if (pa_ && pb_) continue;
+            double *pa = c->pos + 3 * a, *pb = c->pos + 3 * b;
+            double e0 = pa[0] - pb[0], e1 = pa[1] - pb[1], e2 = pa[2] - pb[2];
+            double qd = e0 * e0 + e1 * e1 + e2 * e2;
+            double rest = c->rest[s], c11 = rest * 1.1, ct = rest * tear_thresh;
+            if (qd > ct * ct) c->tear = 1;
+            if (qd > c11 * c11) {
+                double l = sqrt(qd), fac = (l - c11) / l;
+                double fa = pa_ ? 0.0 : (pb_ ? fac : fac * 0.5);
+                double fb = pb_ ? 0.0 : (pa_ ? fac : fac * 0.5);
+                c->n_stretched++;
+                if (c->rec && c->rec_n < c->rec_cap) c->rec[c->rec_n++] = s;
+                if (!pa_) { pa[0] = pa[0] - e0 * fa; pa[1] = pa[1] - e1 * fa; pa[2] = pa[2] - e2 * fa; }
+                if (!pb_) { pb[0] = pb[0] + e0 * fb; pb[1] = pb[1] + e1 * fb; pb[2] = pb[2] + e2 * fb; }
+            }
+        }
+    }
+}
+
+int oracle_update_coloured(OracleCloth *c) {
+    int rc;
+    oracle_phase_gravity(c);
+    if ((rc = oracle_phase_hookes(c))) return rc;
+    oracle_phase_verlet(c);
+    if ((rc = oracle_phase_build_map(c))) return rc;
+    if ((rc = oracle_phase_self_collide_jacobi(c))) return rc;
+    oracle_phase_plane(c);
+    oracle_phase_limit_coloured(c, c->relax_iters);
+    c->n_updates++;
+    return ORACLE_OK;
+}
+
+static int update_in_mode(OracleCloth *c) {
+    return c->mode == ORACLE_MODE_COLOURED ? oracle_update_coloured(c) : oracle_update(c);
+}
+
 int oracle_update_n(OracleCloth *c, int n) {
     for (int i = 0; i < n; i++) {
-        int rc = oracle_update(c);
+        int rc = update_in_mode(c);
         if (rc) return rc;
     }
     return ORACLE_OK;
@@ -549,7 +674,7 @@ int oracle_run_plan(OracleCloth *c, const OraclePlan *plan, int force_grab, int 
         else if ((double)i < iu + iur + ip) oracle_adjust(c, plan->dxr, plan->dyr, 0.0);
         else if ((double)i < iu + iur + ip + igr) { }
         else oracle_release(c);
-        int rc = oracle_update(c);
+        int rc = update_in_mode(c);
         if (rc) return rc;
         nupd++;
         if (c->tear) break; /* :511-514 */

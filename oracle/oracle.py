@@ -75,11 +75,15 @@ def lib():
     L.oracle_cloth_get_springs.argtypes = [vp, i32p, i32p, u8p, dp]
     L.oracle_cloth_set_rest.argtypes = [vp, dp]
     L.oracle_cloth_get_counters.argtypes = [vp, i64p]
+    L.oracle_cloth_set_mode.argtypes = [vp, C.c_int, C.c_int]; L.oracle_cloth_set_mode.restype = None
+    L.oracle_cloth_get_colours.argtypes = [vp, i32p]; L.oracle_cloth_get_colours.restype = None
     for name in ("gravity", "verlet", "plane", "limit"):
         f = getattr(L, "oracle_phase_" + name); f.argtypes = [vp]; f.restype = None
-    for name in ("hookes", "build_map", "self_collide"):
+    for name in ("hookes", "build_map", "self_collide", "self_collide_jacobi"):
         f = getattr(L, "oracle_phase_" + name); f.argtypes = [vp]; f.restype = C.c_int
+    L.oracle_phase_limit_coloured.argtypes = [vp, C.c_int]; L.oracle_phase_limit_coloured.restype = None
     L.oracle_update.argtypes = [vp]; L.oracle_update.restype = C.c_int
+    L.oracle_update_coloured.argtypes = [vp]; L.oracle_update_coloured.restype = C.c_int
     L.oracle_update_n.argtypes = [vp, C.c_int]; L.oracle_update_n.restype = C.c_int
     L.oracle_grab_top.argtypes = [vp, C.c_double, C.c_double, C.c_double]; L.oracle_grab_top.restype = C.c_int
     L.oracle_grab.argtypes = [vp, C.c_double, C.c_double, C.c_double]; L.oracle_grab.restype = C.c_int
@@ -124,12 +128,16 @@ def params_from_cfg(cfg=None):
 
 
 _TIER = {"tier1": 1, "tier2": 2, "tier3": 3, 1: 1, 2: 2, 3: 3}
+_MODE = {"reference_order": 0, "coloured": 1}
 
 
 class OracleCloth(object):
-    """One cloth + gripper, the CPU restatement of Cloth/Gripper/ClothEnv.step."""
+    """One cloth + gripper, the CPU restatement of Cloth/Gripper/ClothEnv.step.
 
-    def __init__(self, params=None, init_type="tier1", noise=None, init_side=True):
+    mode="coloured" makes update() and step_action() run oracle_update_coloured (the specification of the
+    graph-coloured kernels, CLOTHB200_MODE_COLOURED) with max(1, relax_iters) limit passes per update."""
+
+    def __init__(self, params=None, init_type="tier1", noise=None, init_side=True, mode="reference_order", relax_iters=1):
         self.L = lib()
         self.P = params if params is not None else params_from_cfg(None)
         nz = None
@@ -142,6 +150,8 @@ class OracleCloth(object):
             raise ValueError("oracle_cloth_create failed (non-square grid or bad init type)")
         self.N = self.L.oracle_cloth_num_points(self.h)
         self.S = self.L.oracle_cloth_num_springs(self.h)
+        self.mode = mode
+        self.L.oracle_cloth_set_mode(self.h, _MODE[mode], int(relax_iters))
 
     def __del__(self):
         try:
@@ -191,6 +201,10 @@ class OracleCloth(object):
         self.L.oracle_cloth_get_springs(self.h, a, b, t, r)
         return a, b, t, r
 
+    def colours(self):
+        """Colour class 2*kind + parity of every spring (coloured mode), in spring-list order."""
+        out = np.empty(self.S, np.int32); self.L.oracle_cloth_get_colours(self.h, out); return out
+
     def set_rest(self, rest):
         self.L.oracle_cloth_set_rest(self.h, np.ascontiguousarray(rest, np.float64))
 
@@ -208,8 +222,8 @@ class OracleCloth(object):
             raise RuntimeError("oracle error %d" % rc)
         return rc
 
-    def phase(self, name):
-        r = getattr(self.L, "oracle_phase_" + name)(self.h)
+    def phase(self, name, *args):
+        r = getattr(self.L, "oracle_phase_" + name)(self.h, *args)
         if r is not None:
             self._chk(r)
 

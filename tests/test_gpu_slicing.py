@@ -7,7 +7,15 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 
-def _run(dtype, n, sliced, actions, slots=3, q=37, tier=1):
+def queue_parks(c):
+    """Cloths parked by the last sliced launch of BatchedCloth c: the queue counters are the last 16 bytes of
+    sched_scratch (cloth_abi.cu, clothb200_sched_scratch_bytes); tickets issued = n_env + one per park."""
+    qctl = c.sched_scratch[-16:].cpu().numpy().view(np.int32)
+    return int(qctl[1]) - c.n_env
+
+
+def _run(dtype, n, sliced, actions, slots=3, q=37, tier=1, parks=None):
+    """q = 0 keeps the production slice length, swap hysteresis and endgame (CLOTHB200_SLICE and friends)."""
     from gym_cloth_b200 import cfg_path, lib as L
     from gym_cloth_b200.envs import BatchedClothEnv
     lib = L.lib()
@@ -22,6 +30,8 @@ def _run(dtype, n, sliced, actions, slots=3, q=37, tier=1):
         for a in actions:
             obs, rew, done, info = env.step(torch.from_numpy(a).to(env.device, env.torch_dtype))
             c = env.cloth
+            if parks is not None:
+                parks.append(queue_parks(c))
             outs.append({k: v.clone().cpu().numpy() for k, v in dict(pos=c.pos, prev=c.prev, rew=rew, done=done, sim=c.sim_steps, ngrab=c.n_grabbed,
                                                                        flags=c.flags, cov=c.coverage, nss=c.num_sim_steps, mask=c.grab_mask).items()})
     finally:
