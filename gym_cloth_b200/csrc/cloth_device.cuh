@@ -227,6 +227,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     uint32_t *tinfo;         // [TS]   count | (end offset << 16)
     uint16_t *pslot;         // [N]    bucket slot of each point (bit 15: this point allocates the bucket)
     uint16_t *lstA, *lstB;   // [N]    bucket member lists: unordered / index-ordered; lstA later = fix-up work list
+    int *cls;                // [2*NCLS] work-list class counters of the reference-order collision (see NCLS)
     uint32_t *ev;            // [ev_words] stretched-spring queue
     int *misc;               // [16] counters/flags: 0 total, 1 nwork, 2 tear, 3 bad, 4.. scratch
     float2 *kc;              // [8] per spring kind: {rest*1.1, (rest*tear_thresh)^2} (f32, constant rest lengths)
@@ -253,12 +254,18 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
         pslot = reinterpret_cast<uint16_t *>(smem + o);
         ev = reinterpret_cast<uint32_t *>(smem + o); o += ps_bytes > ev_bytes ? ps_bytes : ev_bytes;
         lstA = reinterpret_cast<uint16_t *>(smem + o); o += 2 * (size_t)((N + 7) & ~7);
+        cls = reinterpret_cast<int *>(smem + o); o += cls_bytes();
         lstB = reinterpret_cast<uint16_t *>(smem + o); o += 2 * (size_t)((N + 7) & ~7);
+        if (!cls_bytes()) cls = reinterpret_cast<int *>(lstB);
     }
+    // The class counters sit at the head of lstB when the ordered scatter leaves lstB idle (and the coloured mode has
+    // none).  The unordered scatter writes the index-ordered member lists into lstB while other warps may still read
+    // the counters, and lstB is smaller than the counters on grids of fewer than 136 points: there they get their own.
+    static __host__ __device__ constexpr size_t cls_bytes() { return (ORDERED || COLOURED) ? 0 : 8 * (size_t)NCLS; }
     static __host__ __device__ size_t smem_bytes(int N, int table_size, int ev_words) {
         const size_t ps_bytes = 2 * (size_t)((N + 7) & ~7), ev_bytes = 4 * (size_t)((ev_words + 3) & ~3);
         return sizeof(P4) * (size_t)N * 2 + 8 * (size_t)table_size + 64 + 128 + 64 + (ps_bytes > ev_bytes ? ps_bytes : ev_bytes) +
-               2 * ps_bytes + 16 /* mbarrier */;
+               2 * ps_bytes + cls_bytes() + 16 /* mbarrier */;
     }
 
     __device__ __forceinline__ void sync() {
@@ -347,7 +354,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     // swaps it in after the barrier, when no thread reads old positions any more.
     __device__ __forceinline__ void hooke_verlet() {
         int bad = 0;
-        if (!COLOURED && tid < 2 * NCLS) size_count()[tid] = 0;     // work-list size classes of this substep (lstB is idle here)
+        if (!COLOURED && tid < 2 * NCLS) size_count()[tid] = 0;     // work-list size classes of this substep
         for (int p = tid; p < N; p += NT) {
             const P4 Pp = pos[p];
             if (Pp.w != T(0)) continue;  // pinned: Verlet skips it, its force is never used
@@ -604,9 +611,9 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     //     members    > 32  17-32  11-16  9-10    8   7   6   5   4   3    2
     //     SLOT         -    32     16     10     8   7   6   5   4   3    2
     //     per group    1     1      2      3     4   4   5   6   8  10   16
-    // Class counters, fill counters and the per-class offsets live at the head of lstB, which is idle until
-    // collide_buckets(); hooke_verlet() zeroes them.  The list itself: behind them (ordered scatter: lstB has no other
-    // use) or in the key area (dead after pass 1).
+    // Class counters, fill counters and the per-class offsets live in `cls` (ordered scatter: the head of lstB, which
+    // has no other use); hooke_verlet() zeroes them.  The list itself: behind them (ordered scatter) or in the key area
+    // (dead after pass 1).
     static constexpr int NCLS = 34;                                  // ints reserved per counter block
     static constexpr int NSC = 11;                                   // slot classes
     __device__ __forceinline__ static int cls_of(uint32_t cnt) {
@@ -615,8 +622,8 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     __device__ __forceinline__ static int cls_slot(int c) { return (int)(kSlotClass[c] & 255u); }
     __device__ __forceinline__ static int cls_cap(int c) { return (int)((kSlotClass[c] >> 8) & 255u); }
     __device__ __forceinline__ static int cls_mul(int c) { return (int)(kSlotClass[c] >> 16); }   // ceil(256 / SLOT): lane / SLOT = lane * mul >> 8
-    __device__ __forceinline__ int *size_count() const { return reinterpret_cast<int *>(lstB); }
-    __device__ __forceinline__ int *size_fill() const { return reinterpret_cast<int *>(lstB) + NCLS; }
+    __device__ __forceinline__ int *size_count() const { return cls; }
+    __device__ __forceinline__ int *size_fill() const { return cls + NCLS; }
     __device__ __forceinline__ int *group_off() const { return size_fill() + NSC; }       // first group of each class
     __device__ __forceinline__ int *item_off() const { return size_fill() + 2 * NSC; }    // first work-list index of each class
     __device__ __forceinline__ uint16_t *worklist() const { return ORDERED ? lstB + 4 * NCLS : reinterpret_cast<uint16_t *>(tkey); }

@@ -461,7 +461,13 @@ template <typename T, int NT, int WC, bool RT, bool COL> int launch_step_inst(co
     if (dev < 0 || dev >= CLOTHB200_MAX_DEVICES) return CLOTHB200_ERR_UNSUPPORTED;
     if (smem > configured[dev].load()) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) { set_cuda_error(e, "cudaFuncSetAttribute(smem)"); return CLOTHB200_ERR_UNSUPPORTED; }
+        if (e != cudaSuccess) {
+            // too large for one CTA: refused before anything runs.  The runtime also keeps the error as this thread's
+            // last error, where the next launch check (ours or the caller's) would find it: clear it
+            set_cuda_error(e, "cudaFuncSetAttribute(smem)");
+            cudaGetLastError();
+            return CLOTHB200_ERR_UNSUPPORTED;
+        }
         configured[dev].store(smem);
     }
     if (A.slice > 0) {
@@ -546,6 +552,8 @@ template <typename T> int launch_step(const ClothB200Params &hp, const StepArgs<
 template <typename T> size_t step_smem_bytes(const ClothB200Params &hp) {
     DevParams<T> P;
     make_dev_params(hp, P);
+    // what the reference-order step kernel launched for this grid takes (the ordered scatter needs no counter block)
+    if (P.W == 25 && threads_per_cloth(25) == 128) return ClothCTA<T, 128, 25, true, false>::smem_bytes(P.N, P.table_size, P.ev_words);
     return ClothCTA<T, 128, 0, true, false>::smem_bytes(P.N, P.table_size, P.ev_words);
 }
 

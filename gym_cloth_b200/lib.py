@@ -17,7 +17,11 @@ INIT_TIER = {"tier1": 1, "tier2": 2, "tier3": 3}
 
 
 class ClothB200Error(RuntimeError):
-    pass
+    """`code` is the CLOTHB200_ERR_* return code of the failed library call (None when no call failed)."""
+
+    def __init__(self, msg, code=None):
+        RuntimeError.__init__(self, msg)
+        self.code = code
 
 
 class Params(C.Structure):
@@ -172,7 +176,7 @@ def check(rc, what=""):
         msg = L.clothb200_error_string(rc).decode()
         if rc == -3:
             msg += ": " + L.clothb200_last_cuda_error().decode()
-        raise ClothB200Error("%s failed: %s" % (what or "clothb200 call", msg))
+        raise ClothB200Error("%s failed: %s" % (what or "clothb200 call", msg), rc)
 
 
 def default_params():
