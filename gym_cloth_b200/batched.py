@@ -55,6 +55,9 @@ class BatchedCloth(object):
         self.env_order = None
         self.rest = None
         self.rest_env_stride = 0
+        # per-environment material: None = every cloth runs params' material; else [n_env, 8] float64 on the device,
+        # one ClothB200Physics row per environment (lib.PHYSICS_FIELDS, then two zeros)
+        self.physics = None
         # the parity build always uses the exact per-spring rest lengths; f32 tier-1/3 can use constants
         if exact_rest is None:
             exact_rest = (dtype == torch.float64) or init_type == "tier2"
@@ -172,6 +175,20 @@ class BatchedCloth(object):
             self.rest[env] = t
         self.exact_rest = True
 
+    def set_physics(self, envs=None, **fields):
+        """Per-environment material: set the given lib.PHYSICS_FIELDS (scalars or one value per selected environment)
+        for all (or the given) environments.  The first call starts every row from params' values.  Rows are not
+        checked here: the kernels treat a row with a non-finite value or density <= 0 as a bad action (BADSTATE)."""
+        unknown = set(fields) - set(_l.PHYSICS_FIELDS)
+        if unknown:
+            raise TypeError("unknown physics fields: %s" % sorted(unknown))
+        if self.physics is None:
+            row = [getattr(self.P, k) for k in _l.PHYSICS_FIELDS] + [0.0, 0.0]
+            self.physics = torch.tensor([row], dtype=torch.float64, device=self.device).repeat(self.n_env, 1).contiguous()
+        sel = slice(None) if envs is None else torch.as_tensor(np.asarray(envs, np.int64), device=self.device)
+        for k, v in fields.items():
+            self.physics[sel, _l.PHYSICS_FIELDS.index(k)] = torch.as_tensor(np.asarray(v, np.float64), device=self.device)
+
     # ------------------------------------------------------------------ state access
     def set_state(self, pos3, prev3, pinned=None, grabbed=None, env=None, tear=False):
         """Load one state (N x 3 arrays, pinned [N] bool, grabbed = index list with multiplicity)
@@ -205,6 +222,10 @@ class BatchedCloth(object):
     def update(self, n_updates=1, measure=False):
         """n x Cloth.update() (cloth.pyx:169-214)."""
         io = self.io(measure=measure, bookkeeping=False, obs=False, grab_mask=False)
+        if self.physics is not None:
+            _l.check(self._f("clothb200_update_n_phys")(C.byref(self.P), self.mode, self.n_env, int(n_updates), C.byref(io),
+                                                       _ptr(self.physics), self.stream), "update_n_phys")
+            return
         _l.check(self._f("clothb200_update_n")(C.byref(self.P), self.mode, self.n_env, int(n_updates), C.byref(io),
                                               self.stream), "update_n")
 
@@ -222,6 +243,10 @@ class BatchedCloth(object):
             self.plans.copy_(host)
             plans = self.plans
         io = self.io(measure=measure, bookkeeping=not initialize, obs=obs)
+        if self.physics is not None:
+            _l.check(self._f("clothb200_step_plans_phys")(C.byref(self.P), self.mode, self.n_env, _ptr(plans), C.byref(io),
+                                                         int(initialize), _ptr(self.physics), self.stream), "step_plans_phys")
+            return
         _l.check(self._f("clothb200_step_plans")(C.byref(self.P), self.mode, self.n_env, _ptr(plans), C.byref(io),
                                                 int(initialize), self.stream), "step_plans")
 
@@ -229,6 +254,11 @@ class BatchedCloth(object):
         """actions: device tensor [n_env, 4] of this cloth's dtype, env.step format.  Decode on device."""
         assert actions.is_cuda and actions.dtype == self.dtype and actions.is_contiguous()
         io = self.io(measure=measure, bookkeeping=not initialize, obs=obs)
+        if self.physics is not None:
+            _l.check(self._f("clothb200_step_actions_phys")(C.byref(self.P), self.mode, self.n_env, _ptr(actions),
+                                                           _ptr(self.plans), C.byref(io), int(initialize), _ptr(self.physics),
+                                                           self.stream), "step_actions_phys")
+            return
         _l.check(self._f("clothb200_step_actions")(C.byref(self.P), self.mode, self.n_env, _ptr(actions), _ptr(self.plans),
                                                   C.byref(io), int(initialize), self.stream), "step_actions")
 
@@ -238,6 +268,12 @@ class BatchedCloth(object):
         a = np.ascontiguousarray(actions, np.float64)
         io = self.io(measure=True, bookkeeping=not initialize, obs=("obs" in out))
         g = lambda k: C.c_void_p(out[k].ctypes.data if isinstance(out[k], np.ndarray) else out[k].data_ptr()) if k in out else None
+        if self.physics is not None:
+            _l.check(self._f("clothb200_step_host_phys")(C.byref(self.P), self.mode, self.n_env, a.ctypes.data, C.byref(io),
+                                                        int(initialize), g("obs"), g("reward"), g("done"), g("coverage"),
+                                                        g("variance_inv"), g("flags"), g("sim_steps"), _ptr(self.physics),
+                                                        self.stream), "step_host_phys")
+            return
         _l.check(self._f("clothb200_step_host")(C.byref(self.P), self.mode, self.n_env, a.ctypes.data, C.byref(io), int(initialize),
                                                g("obs"), g("reward"), g("done"), g("coverage"), g("variance_inv"), g("flags"),
                                                g("sim_steps"), self.stream), "step_host")

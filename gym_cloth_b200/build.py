@@ -5,7 +5,8 @@
 
 Translation units, compiled in parallel: cloth_f32.cu (production entry points + renderer), cloth_f64.cu (parity
 build, -fmad=false so that every operator is one rounded IEEE operation), cloth_abi.cu (extern "C" surface) and
-cloth_inst.cu six times (the step kernel per scalar type and compile-time grid width).
+cloth_inst.cu twelve times (the step kernel per scalar type, compile-time grid width, and batch or per-environment
+material).
 """
 import os
 import subprocess
@@ -22,11 +23,14 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relax
 # f64 (parity): no FMA contraction, IEEE everything.
 F32 = ["-ftz=true", "-prec-div=false", "-prec-sqrt=false"]
 F64 = ["-fmad=false"]
-# (source, object name, flags); cloth_inst.cu holds the step kernel for one (scalar type, grid width) pair
+# (source, object name, flags); cloth_inst.cu holds the step kernel for one (scalar type, grid width) pair, with the
+# batch's material or (cloth_inst_phys_*) with per-environment material rows
 UNITS = [("cloth_f32.cu", "cloth_f32.o", F32), ("cloth_f64.cu", "cloth_f64.o", F64), ("cloth_abi.cu", "cloth_abi.o", [])]
 for _t, _sfx, _fl in (("float", "f32", F32), ("double", "f64", F64)):
     for _w in (25, 0, 64):
         UNITS.append(("cloth_inst.cu", "cloth_inst_%s_w%d.o" % (_sfx, _w), _fl + ["-DCLOTH_T=%s" % _t, "-DCLOTH_INSTANTIATE_WC=%d" % _w]))
+        UNITS.append(("cloth_inst.cu", "cloth_inst_phys_%s_w%d.o" % (_sfx, _w),
+                      _fl + ["-DCLOTH_T=%s" % _t, "-DCLOTH_INSTANTIATE_WC=%d" % _w, "-DCLOTH_INSTANTIATE_PHYS=1"]))
 
 
 def _newest_src():
@@ -48,7 +52,10 @@ IEEE = ["-DCLOTHB200_F32_REFERENCE_FORMS", "-ftz=false", "-prec-div=true", "-pre
 UNITS_IEEE = [("cloth_f32.cu", "ieee_cloth_f32.o", IEEE), ("cloth_f64.cu", "cloth_f64.o", None), ("cloth_abi.cu", "cloth_abi.o", None)]
 for _w in (25, 0, 64):
     UNITS_IEEE.append(("cloth_inst.cu", "ieee_cloth_inst_f32_w%d.o" % _w, IEEE + ["-DCLOTH_T=float", "-DCLOTH_INSTANTIATE_WC=%d" % _w]))
+    UNITS_IEEE.append(("cloth_inst.cu", "ieee_cloth_inst_phys_f32_w%d.o" % _w,
+                       IEEE + ["-DCLOTH_T=float", "-DCLOTH_INSTANTIATE_WC=%d" % _w, "-DCLOTH_INSTANTIATE_PHYS=1"]))
     UNITS_IEEE.append(("cloth_inst.cu", "cloth_inst_f64_w%d.o" % _w, None))
+    UNITS_IEEE.append(("cloth_inst.cu", "cloth_inst_phys_f64_w%d.o" % _w, None))
 
 
 def build_ieee(force=False, verbose=False):

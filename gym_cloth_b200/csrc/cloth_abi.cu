@@ -111,8 +111,8 @@ const uint32_t *get_sweep_table(int W, int *levels, int *lw) {
 }
 // typed entry points (cloth_f32.cu / cloth_f64.cu)
 #define DECL_TYPED(SFX, T)                                                                                                               \
-    int step_plans_##SFX(const ClothB200Params *, int, int, const ClothB200Plan *, const ClothB200Step *, int, cudaStream_t);            \
-    int update_n_##SFX(const ClothB200Params *, int, int, int, const ClothB200Step *, cudaStream_t);                                     \
+    int step_plans_##SFX(const ClothB200Params *, int, int, const ClothB200Plan *, const ClothB200Step *, int, const ClothB200Physics *, cudaStream_t); \
+    int update_n_##SFX(const ClothB200Params *, int, int, int, const ClothB200Step *, const ClothB200Physics *, cudaStream_t);          \
     int grab_top_##SFX(const ClothB200Params *, int, const double *, double, const ClothB200Step *, cudaStream_t);                       \
     int measure_##SFX(const ClothB200Params *, int, const ClothB200Step *, cudaStream_t);                                                \
     int decode_actions_##SFX(const ClothB200Params *, int, const T *, ClothB200Plan *, cudaStream_t);                                    \
@@ -120,7 +120,8 @@ const uint32_t *get_sweep_table(int W, int *levels, int *lw) {
     int gripper_adjust_##SFX(int, int, double, double, double, T *, T *, cudaStream_t);                                                  \
     int gripper_release_##SFX(int, int, T *, T *, cudaStream_t);                                                                         \
     int render_##SFX(const ClothB200Params *, const ClothB200Scene *, const ClothB200SceneEnv *, int, const T *, int, uint8_t *, float *, unsigned *, cudaStream_t); \
-    size_t step_smem_##SFX(const ClothB200Params *);
+    size_t step_smem_##SFX(const ClothB200Params *);                                                                                    \
+    int kernel_info_##SFX(const ClothB200Params *, int, int, int, int *);
 DECL_TYPED(f32, float)
 DECL_TYPED(f64, double)
 
@@ -196,6 +197,44 @@ struct HostScratch {
     }
 };
 static thread_local HostScratch g_scratch;
+
+// Per-environment material rows of the *_phys_* entry points (launch_step): one device buffer per thread, grown when a
+// call needs more and reused by the next call, so that the many small update_n calls of a reset allocate nothing.  An
+// event recorded behind each call's step kernel orders reuse: a call on another stream waits for it before its derive
+// kernel overwrites the rows (on the same stream the wait is already implied).
+struct MaterialRows {
+    void *dev = nullptr;
+    size_t cap = 0;
+    int device = -1;
+    cudaEvent_t done = nullptr;
+};
+static thread_local MaterialRows g_rows;
+
+void *material_rows(size_t bytes, cudaStream_t st, int *rc) {
+    int cur = 0;
+    cudaGetDevice(&cur);
+    MaterialRows &m = g_rows;
+    if (m.device != cur || bytes > m.cap) {
+        if (m.done) { cudaEventSynchronize(m.done); cudaEventDestroy(m.done); }   // the old rows may still be read
+        if (m.dev) cudaFree(m.dev);
+        m = MaterialRows();
+        size_t cap = 8192;
+        while (cap < bytes) cap <<= 1;
+        *rc = check_cuda(cudaMalloc(&m.dev, cap), "cudaMalloc(material rows)");
+        if (*rc == CLOTHB200_OK) *rc = check_cuda(cudaEventCreateWithFlags(&m.done, cudaEventDisableTiming), "cudaEventCreate(material rows)");
+        if (*rc) {
+            if (m.dev) cudaFree(m.dev);
+            m = MaterialRows();
+            cudaGetLastError();
+            return nullptr;
+        }
+        m.cap = cap; m.device = cur;
+        return m.dev;
+    }
+    *rc = check_cuda(cudaStreamWaitEvent(st, m.done, 0), "cudaStreamWaitEvent(material rows)");
+    return *rc ? nullptr : m.dev;
+}
+int material_rows_release(cudaStream_t st) { return check_cuda(cudaEventRecord(g_rows.done, st), "cudaEventRecord(material rows)"); }
 
 // ---- microbenchmarks: this GPU's shared-memory bandwidth and FP32 FMA rate (roofline denominators) ----
 __global__ void __launch_bounds__(1024) smem_bw_kernel(int iters, float *sink) {
@@ -295,6 +334,7 @@ const char *clothb200_last_cuda_error(void) { return g_cuda_err.c_str(); }
 size_t clothb200_sizeof_params(void) { return sizeof(ClothB200Params); }
 size_t clothb200_sizeof_plan(void) { return sizeof(ClothB200Plan); }
 size_t clothb200_sizeof_step(void) { return sizeof(ClothB200Step); }
+size_t clothb200_sizeof_physics(void) { return sizeof(ClothB200Physics); }
 int clothb200_debug_set_slicing(int resident_ctas, int slice_substeps) {
     g_force_slots = resident_ctas > 0 ? resident_ctas : 0;
     g_force_slice = slice_substeps > 0 ? slice_substeps : 0;
@@ -318,6 +358,20 @@ int clothb200_device_info(int device, int *sm_count, int *cc_major, int *cc_mino
     if (cc_major) *cc_major = pr.major;
     if (cc_minor) *cc_minor = pr.minor;
     if (smem_per_sm) *smem_per_sm = (int)pr.sharedMemPerMultiprocessor;
+    return CLOTHB200_OK;
+}
+
+int clothb200_step_kernel_info(const ClothB200Params *p, int is_f64, int mode, int rest_table, int per_env_physics, int *ctas_per_sm,
+                               int *registers, int *local_bytes, int *smem_bytes) {
+    if (!p) return CLOTHB200_ERR_ARG;
+    if (mode != CLOTHB200_MODE_REFERENCE_ORDER && mode != CLOTHB200_MODE_COLOURED) return CLOTHB200_ERR_UNSUPPORTED;
+    int out[4] = {0, 0, 0, 0};
+    const int rc = is_f64 ? kernel_info_f64(p, mode, rest_table, per_env_physics, out) : kernel_info_f32(p, mode, rest_table, per_env_physics, out);
+    if (rc) return rc;
+    if (ctas_per_sm) *ctas_per_sm = out[0];
+    if (registers) *registers = out[1];
+    if (local_bytes) *local_bytes = out[2];
+    if (smem_bytes) *smem_bytes = out[3];
     return CLOTHB200_OK;
 }
 
@@ -411,22 +465,33 @@ int clothb200_decode_actions_host(const ClothB200Params *P, int n_env, const dou
 int clothb200_decode_actions_f32(const ClothB200Params *p, int n, const float *a, ClothB200Plan *plans, void *st) { return decode_actions_f32(p, n, a, plans, (cudaStream_t)st); }
 int clothb200_decode_actions_f64(const ClothB200Params *p, int n, const double *a, ClothB200Plan *plans, void *st) { return decode_actions_f64(p, n, a, plans, (cudaStream_t)st); }
 
-int clothb200_step_plans_f32(const ClothB200Params *p, int mode, int n, const ClothB200Plan *plans, const ClothB200Step *io, int init, void *st) { return step_plans_f32(p, mode, n, plans, io, init, (cudaStream_t)st); }
-int clothb200_step_plans_f64(const ClothB200Params *p, int mode, int n, const ClothB200Plan *plans, const ClothB200Step *io, int init, void *st) { return step_plans_f64(p, mode, n, plans, io, init, (cudaStream_t)st); }
+// physics == NULL: the batch's material (the plain entry points below are these with NULL)
+int clothb200_step_plans_phys_f32(const ClothB200Params *p, int mode, int n, const ClothB200Plan *plans, const ClothB200Step *io, int init, const ClothB200Physics *ph, void *st) { return step_plans_f32(p, mode, n, plans, io, init, ph, (cudaStream_t)st); }
+int clothb200_step_plans_phys_f64(const ClothB200Params *p, int mode, int n, const ClothB200Plan *plans, const ClothB200Step *io, int init, const ClothB200Physics *ph, void *st) { return step_plans_f64(p, mode, n, plans, io, init, ph, (cudaStream_t)st); }
+int clothb200_step_plans_f32(const ClothB200Params *p, int mode, int n, const ClothB200Plan *plans, const ClothB200Step *io, int init, void *st) { return clothb200_step_plans_phys_f32(p, mode, n, plans, io, init, nullptr, st); }
+int clothb200_step_plans_f64(const ClothB200Params *p, int mode, int n, const ClothB200Plan *plans, const ClothB200Step *io, int init, void *st) { return clothb200_step_plans_phys_f64(p, mode, n, plans, io, init, nullptr, st); }
 
-int clothb200_step_actions_f32(const ClothB200Params *p, int mode, int n, const float *actions, ClothB200Plan *scratch, const ClothB200Step *io, int init, void *st) {
+int clothb200_step_actions_phys_f32(const ClothB200Params *p, int mode, int n, const float *actions, ClothB200Plan *scratch, const ClothB200Step *io, int init, const ClothB200Physics *ph, void *st) {
     int rc = decode_actions_f32(p, n, actions, scratch, (cudaStream_t)st);
     if (rc) return rc;
-    return step_plans_f32(p, mode, n, scratch, io, init, (cudaStream_t)st);
+    return step_plans_f32(p, mode, n, scratch, io, init, ph, (cudaStream_t)st);
 }
-int clothb200_step_actions_f64(const ClothB200Params *p, int mode, int n, const double *actions, ClothB200Plan *scratch, const ClothB200Step *io, int init, void *st) {
+int clothb200_step_actions_phys_f64(const ClothB200Params *p, int mode, int n, const double *actions, ClothB200Plan *scratch, const ClothB200Step *io, int init, const ClothB200Physics *ph, void *st) {
     int rc = decode_actions_f64(p, n, actions, scratch, (cudaStream_t)st);
     if (rc) return rc;
-    return step_plans_f64(p, mode, n, scratch, io, init, (cudaStream_t)st);
+    return step_plans_f64(p, mode, n, scratch, io, init, ph, (cudaStream_t)st);
+}
+int clothb200_step_actions_f32(const ClothB200Params *p, int mode, int n, const float *actions, ClothB200Plan *scratch, const ClothB200Step *io, int init, void *st) {
+    return clothb200_step_actions_phys_f32(p, mode, n, actions, scratch, io, init, nullptr, st);
+}
+int clothb200_step_actions_f64(const ClothB200Params *p, int mode, int n, const double *actions, ClothB200Plan *scratch, const ClothB200Step *io, int init, void *st) {
+    return clothb200_step_actions_phys_f64(p, mode, n, actions, scratch, io, init, nullptr, st);
 }
 
-int clothb200_update_n_f32(const ClothB200Params *p, int mode, int n, int k, const ClothB200Step *io, void *st) { return update_n_f32(p, mode, n, k, io, (cudaStream_t)st); }
-int clothb200_update_n_f64(const ClothB200Params *p, int mode, int n, int k, const ClothB200Step *io, void *st) { return update_n_f64(p, mode, n, k, io, (cudaStream_t)st); }
+int clothb200_update_n_phys_f32(const ClothB200Params *p, int mode, int n, int k, const ClothB200Step *io, const ClothB200Physics *ph, void *st) { return update_n_f32(p, mode, n, k, io, ph, (cudaStream_t)st); }
+int clothb200_update_n_phys_f64(const ClothB200Params *p, int mode, int n, int k, const ClothB200Step *io, const ClothB200Physics *ph, void *st) { return update_n_f64(p, mode, n, k, io, ph, (cudaStream_t)st); }
+int clothb200_update_n_f32(const ClothB200Params *p, int mode, int n, int k, const ClothB200Step *io, void *st) { return clothb200_update_n_phys_f32(p, mode, n, k, io, nullptr, st); }
+int clothb200_update_n_f64(const ClothB200Params *p, int mode, int n, int k, const ClothB200Step *io, void *st) { return clothb200_update_n_phys_f64(p, mode, n, k, io, nullptr, st); }
 
 int clothb200_grab_top_f32(const ClothB200Params *p, int n, const double *xy, double r, const ClothB200Step *io, void *st) { return grab_top_f32(p, n, xy, r, io, (cudaStream_t)st); }
 int clothb200_grab_top_f64(const ClothB200Params *p, int n, const double *xy, double r, const ClothB200Step *io, void *st) { return grab_top_f64(p, n, xy, r, io, (cudaStream_t)st); }
@@ -486,7 +551,7 @@ int clothb200_measure_f64(const ClothB200Params *p, int n, const ClothB200Step *
     if (rc) return rc;                                                                                                                   \
     rc = check_cuda(cudaMemcpyAsync(g_scratch.dev, g_scratch.pinned, sizeof(ClothB200Plan) * (size_t)n, cudaMemcpyHostToDevice, s), "H2D plans"); \
     if (rc) return rc;                                                                                                                   \
-    rc = step_plans_##SFX(p, mode, n, g_scratch.dev, io, initialize, s);                                                                 \
+    rc = step_plans_##SFX(p, mode, n, g_scratch.dev, io, initialize, physics, s);                                                        \
     if (rc) return rc;                                                                                                                   \
     const size_t N3 = (size_t)3 * p->num_width_points * p->num_height_points;                                                            \
     if (obs) rc |= check_cuda(cudaMemcpyAsync(obs, io->obs, sizeof(T) * N3 * n, cudaMemcpyDeviceToHost, s), "D2H obs");                  \
@@ -499,15 +564,25 @@ int clothb200_measure_f64(const ClothB200Params *p, int n, const ClothB200Step *
     if (rc) return CLOTHB200_ERR_CUDA;                                                                                                   \
     return check_cuda(cudaStreamSynchronize(s), "cudaStreamSynchronize");
 
+int clothb200_step_host_phys_f32(const ClothB200Params *p, int mode, int n, const double *actions, const ClothB200Step *io, int initialize,
+                                 float *obs, double *reward, int32_t *done, double *coverage, double *variance_inv, int32_t *flags,
+                                 int32_t *sim_steps, const ClothB200Physics *physics, void *st) {
+    STEP_HOST_BODY(f32, float)
+}
+int clothb200_step_host_phys_f64(const ClothB200Params *p, int mode, int n, const double *actions, const ClothB200Step *io, int initialize,
+                                 double *obs, double *reward, int32_t *done, double *coverage, double *variance_inv, int32_t *flags,
+                                 int32_t *sim_steps, const ClothB200Physics *physics, void *st) {
+    STEP_HOST_BODY(f64, double)
+}
 int clothb200_step_host_f32(const ClothB200Params *p, int mode, int n, const double *actions, const ClothB200Step *io, int initialize,
                             float *obs, double *reward, int32_t *done, double *coverage, double *variance_inv, int32_t *flags,
                             int32_t *sim_steps, void *st) {
-    STEP_HOST_BODY(f32, float)
+    return clothb200_step_host_phys_f32(p, mode, n, actions, io, initialize, obs, reward, done, coverage, variance_inv, flags, sim_steps, nullptr, st);
 }
 int clothb200_step_host_f64(const ClothB200Params *p, int mode, int n, const double *actions, const ClothB200Step *io, int initialize,
                             double *obs, double *reward, int32_t *done, double *coverage, double *variance_inv, int32_t *flags,
                             int32_t *sim_steps, void *st) {
-    STEP_HOST_BODY(f64, double)
+    return clothb200_step_host_phys_f64(p, mode, n, actions, io, initialize, obs, reward, done, coverage, variance_inv, flags, sim_steps, nullptr, st);
 }
 
 static int time_kernel(void (*launch)(int, float *, cudaStream_t), int iters, cudaStream_t s, float *ms_out) {

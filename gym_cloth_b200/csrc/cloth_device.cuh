@@ -72,6 +72,43 @@ template <typename T> struct DevParams {
     int force_grab;              // cfg env.force_grab: grow the grip radius by 0.02 until something is gripped (cloth_env.py:434-444)
 };
 
+// The material constants of one cloth: what density, ks, damping, plane_friction, tear_thresh and gravity become.
+// DevParams carries the batch's; the per-environment step kernel reads one row of these per cloth instead, through the
+// read-only path.  The fields Hooke/Verlet reads every substep come first (44 of the 80 bytes of an f32 row; rows are not
+// padded to 64 bytes, so these span two or three 32-byte sectors, loaded once per CTA into L1).
+template <typename T> struct DevMaterial {
+    T mg, kk_struct, kk_bend, dsdm, damp;
+    T kkrest_k[6];
+    T fric1, tear_thresh;
+    T limit_c2_k[6];
+    int valid;                   // 0: a non-finite value or density <= 0 (the cloth is not stepped, BADSTATE)
+};
+
+// cloth.pyx:175-186, 240-241: the constants in double as the reference derives them, then rounded to T once; the
+// per-kind products are formed in T from those.  The one place this arithmetic lives (make_dev_params and the
+// per-environment rows both call it), so the same material gives the same bits either way.
+template <typename T>
+__host__ __device__ inline void derive_material(double density, double ks, double damping, double plane_friction, double tear_thresh,
+                                                double gravity, int W, int H, double frames_per_sec, int simulation_steps,
+                                                const T *rest_k, DevMaterial<T> &m) {
+    const double mass = density / W / H;
+    const double delta_t = 1.0 / frames_per_sec / simulation_steps;
+    m.mg = (T)(mass * gravity);
+    m.kk_struct = (T)(ks * 1.0);
+    m.kk_bend = (T)(ks * 0.2);
+    m.dsdm = (T)((delta_t * delta_t) / mass);
+    m.damp = (T)(1.0 - damping / 100.0);
+    m.fric1 = (T)(1. - plane_friction);
+    m.tear_thresh = (T)tear_thresh;
+    for (int k = 0; k < 6; k++) {
+        m.kkrest_k[k] = (k >= 4 ? m.kk_bend : m.kk_struct) * rest_k[k];
+        const T a = rest_k[k] * T(1.1), b = rest_k[k] * m.tear_thresh, c = a < b ? a : b;    // ClothCTA::limit_c
+        m.limit_c2_k[k] = c * c;
+    }
+    m.valid = isfinite(density) && isfinite(ks) && isfinite(damping) && isfinite(plane_friction) && isfinite(tear_thresh) &&
+              isfinite(gravity) && density > 0;
+}
+
 template <typename T> struct StepArgs {
     T *pos, *prev;
     const T *rest;
@@ -106,6 +143,7 @@ template <typename T> struct StepArgs {
     int *qctl;                   // [0] tickets taken, [1] tickets issued, [2] cloths finished
     int *progress, *ngrab_s;     // [qcap] per item: substeps done, number of gripped points
     float *cycles_s;             // [qcap] per item: SM cycles spent so far
+    const DevMaterial<T> *mat;   // [n_env] by launch position (item): per-environment material (the PHYS kernels only)
 };
 
 enum { KMODE_STEP = 0, KMODE_UPDATE = 1, KMODE_GRAB = 2, KMODE_MEASURE = 3 };
@@ -207,7 +245,7 @@ static __device__ __constant__ uint32_t kSlotClass[11] = {
 #define CLOTH_KEY_EMPTY 0x7fffffff
 #define CLOTH_FIRST_NONE 0x7ffffffe
 
-template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> struct ClothCTA {
+template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bool PHYS = false> struct ClothCTA {
     typedef typename V4<T>::type P4;
     static constexpr int NWARPS = NT / 32;
     // f32 production math (rsqrt / squared-distance forms of the reference's expressions); the f64 build evaluates the
@@ -232,14 +270,15 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     int *misc;               // [16] counters/flags: 0 total, 1 nwork, 2 tear, 3 bad, 4.. scratch
     float2 *kc;              // [8] per spring kind: {rest*1.1, (rest*tear_thresh)^2} (f32, constant rest lengths)
     const T *rest;           // rest table of this env (REST_TABLE)
+    const DevMaterial<T> *mat;   // material row of this env (PHYS), read through the read-only path where a phase uses it
     int rot;                 // blockIdx-derived rotation of the warp roles (spreads serial phases over the 4 SM sub-partitions)
     long long *pacc;         // [16] smem: thread 0's cycles per phase + event counters when profiling
     long long plast;
     bool prof_on;
 
-    __device__ ClothCTA(const DevParams<T> &P_, unsigned char *smem, const T *rest_)
+    __device__ ClothCTA(const DevParams<T> &P_, unsigned char *smem, const T *rest_, const DevMaterial<T> *mat_ = nullptr)
         : P(P_), W(WC ? WC : P_.W), H(WC ? WC : P_.H), N(WC ? WC * WC : P_.N), tid(threadIdx.x), lane(threadIdx.x & 31),
-          warp(threadIdx.x >> 5), rest(rest_), rot((int)blockIdx.x), plast(0), prof_on(false) {
+          warp(threadIdx.x >> 5), rest(rest_), mat(mat_), rot((int)blockIdx.x), plast(0), prof_on(false) {
         size_t o = 0;
         pos = reinterpret_cast<P4 *>(smem + o); o += sizeof(P4) * (size_t)N;
         prev = reinterpret_cast<P4 *>(smem + o); o += sizeof(P4) * (size_t)N;
@@ -292,6 +331,17 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
         T hi = k == 3 ? v[3] : (k == 4 ? v[4] : v[5]);
         return k < 3 ? lo : hi;
     }
+    // ---- material constants: the launch's (P), or this cloth's row in the per-environment variant ----
+    __device__ __forceinline__ T mg() const { if constexpr (PHYS) return __ldg(&mat->mg); else return P.mg; }
+    __device__ __forceinline__ T kk_struct() const { if constexpr (PHYS) return __ldg(&mat->kk_struct); else return P.kk_struct; }
+    __device__ __forceinline__ T kk_bend() const { if constexpr (PHYS) return __ldg(&mat->kk_bend); else return P.kk_bend; }
+    __device__ __forceinline__ T dsdm() const { if constexpr (PHYS) return __ldg(&mat->dsdm); else return P.dsdm; }
+    __device__ __forceinline__ T damp() const { if constexpr (PHYS) return __ldg(&mat->damp); else return P.damp; }
+    __device__ __forceinline__ T fric1() const { if constexpr (PHYS) return __ldg(&mat->fric1); else return P.fric1; }
+    __device__ __forceinline__ T tear_thresh() const { if constexpr (PHYS) return __ldg(&mat->tear_thresh); else return P.tear_thresh; }
+    __device__ __forceinline__ T kkrest_k(int k) const { if constexpr (PHYS) return __ldg(&mat->kkrest_k[k]); else return P.kkrest_k[k]; }
+    __device__ __forceinline__ T limit_c2_k(int k) const { if constexpr (PHYS) return __ldg(&mat->limit_c2_k[k]); else return P.limit_c2_k[k]; }
+
     __device__ __forceinline__ T rest_of(int q, int k) const {
         if (REST_TABLE) return __ldg(rest + q * 6 + k);
         return sel6(P.rest_k, k);
@@ -299,9 +349,9 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     // kk * rest of spring (q, k): a launch constant unless the cloth carries its own rest lengths
     __device__ __forceinline__ T kkrest_of(int q, int k, T kk) const {
         if (REST_TABLE || !FAST) return kk * rest_of(q, k);
-        return P.kkrest_k[k];
+        return kkrest_k(k);
     }
-    __device__ __forceinline__ T kk_of(int k) const { return k >= 4 ? P.kk_bend : P.kk_struct; }
+    __device__ __forceinline__ T kk_of(int k) const { return k >= 4 ? kk_bend() : kk_struct(); }
 
     // ---- distance predicates ----
     // f32 build: squared-distance forms (no sqrt).  f64 build: the reference's exact `fastnorm(...) <op> c`
@@ -327,7 +377,8 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     // ---- Hooke (cloth.pyx:221-237) gathered per point + Verlet (cloth.pyx:239-256) ----
     // One spring's contribution to point p, selected without branches so that the 12 neighbour loads and
     // the 12 independent force evaluations of a point can overlap.  SIGN=+1: p is ptA, -1: p is ptB.
-    template <int SIGN>
+    // Z_RN: fz -= fm*d2 as a rounded product and a rounded difference (see hooke_verlet)
+    template <int SIGN, bool Z_RN = false>
     __device__ __forceinline__ void add_spring(bool valid, const P4 &Pa, const P4 &Pb, T kk, T rst, T kkrst, T &fx, T &fy, T &fz, int &bad) {
         const T d0 = Pb.x - Pa.x, d1 = Pb.y - Pa.y, d2 = Pb.z - Pa.z;
         const T q = d0 * d0 + d1 * d1 + d2 * d2;
@@ -337,6 +388,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
             // positions, which commit_and_hash() reports as BADSTATE (the reference raises ZeroDivisionError here)
             fm = valid ? kk - kkrst * rsqrtf((float)q) : T(0);
             if (SIGN > 0) { fx += fm * d0; fy += fm * d1; fz += fm * d2; }
+            else if constexpr (Z_RN) { fx -= fm * d0; fy -= fm * d1; fz = __fsub_rn(fz, __fmul_rn(fm, d2)); }
             else { fx -= fm * d0; fy -= fm * d1; fz -= fm * d2; }
             return;
         }
@@ -368,26 +420,29 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
             const P4 B3 = pos[u3 ? p + W : p], B4 = pos[u4 ? p + W + 1 : p], B5 = pos[u5 ? p + 2 * W : p];
             const P4 Q = prev[p];
             // _reset_gravity: f = 0 then f += (0,0,mg)
-            T fx = T(0) + T(0), fy = T(0) + T(0), fz = T(0) + P.mg;
-            // springs created by p (p is ptB, ptB.add_force(-F)), creation order k = 0..5
-            add_spring<-1>(v0, A0, Pp, P.kk_struct, rest_of(p, 0), kkrest_of(p, 0, P.kk_struct), fx, fy, fz, bad);
-            add_spring<-1>(v1, A1, Pp, P.kk_struct, rest_of(p, 1), kkrest_of(p, 1, P.kk_struct), fx, fy, fz, bad);
-            add_spring<-1>(v2, A2, Pp, P.kk_struct, rest_of(p, 2), kkrest_of(p, 2, P.kk_struct), fx, fy, fz, bad);
-            add_spring<-1>(v3, A3, Pp, P.kk_struct, rest_of(p, 3), kkrest_of(p, 3, P.kk_struct), fx, fy, fz, bad);
-            add_spring<-1>(v4, A4, Pp, P.kk_bend, rest_of(p, 4), kkrest_of(p, 4, P.kk_bend), fx, fy, fz, bad);
-            add_spring<-1>(v5, A5, Pp, P.kk_bend, rest_of(p, 5), kkrest_of(p, 5, P.kk_bend), fx, fy, fz, bad);
+            T fx = T(0) + T(0), fy = T(0) + T(0), fz = T(0) + mg();
+            // springs created by p (p is ptB, ptB.add_force(-F)), creation order k = 0..5.  In the f32 kernels with the
+            // batch's material ptxas keeps the first spring's z product apart from mg (FMUL + FADD, not FFMA); with mg
+            // read from the cloth's row it would fuse them, so the per-environment variant rounds both explicitly: the
+            // same material gives the same bits in either kernel
+            add_spring<-1, PHYS && FAST>(v0, A0, Pp, kk_struct(), rest_of(p, 0), kkrest_of(p, 0, kk_struct()), fx, fy, fz, bad);
+            add_spring<-1>(v1, A1, Pp, kk_struct(), rest_of(p, 1), kkrest_of(p, 1, kk_struct()), fx, fy, fz, bad);
+            add_spring<-1>(v2, A2, Pp, kk_struct(), rest_of(p, 2), kkrest_of(p, 2, kk_struct()), fx, fy, fz, bad);
+            add_spring<-1>(v3, A3, Pp, kk_struct(), rest_of(p, 3), kkrest_of(p, 3, kk_struct()), fx, fy, fz, bad);
+            add_spring<-1>(v4, A4, Pp, kk_bend(), rest_of(p, 4), kkrest_of(p, 4, kk_bend()), fx, fy, fz, bad);
+            add_spring<-1>(v5, A5, Pp, kk_bend(), rest_of(p, 5), kkrest_of(p, 5, kk_bend()), fx, fy, fz, bad);
             // springs created by later points in which p is ptA, in creation order:
             // q = p+1 (k=1), p+2 (k=5), p+W-1 (k=3), p+W (k=0), p+W+1 (k=2), p+2W (k=4)
-            add_spring<1>(u0, Pp, B0, P.kk_struct, rest_of(u0 ? p + 1 : p, 1), kkrest_of(u0 ? p + 1 : p, 1, P.kk_struct), fx, fy, fz, bad);
-            add_spring<1>(u1, Pp, B1, P.kk_bend, rest_of(u1 ? p + 2 : p, 5), kkrest_of(u1 ? p + 2 : p, 5, P.kk_bend), fx, fy, fz, bad);
-            add_spring<1>(u2, Pp, B2, P.kk_struct, rest_of(u2 ? p + W - 1 : p, 3), kkrest_of(u2 ? p + W - 1 : p, 3, P.kk_struct), fx, fy, fz, bad);
-            add_spring<1>(u3, Pp, B3, P.kk_struct, rest_of(u3 ? p + W : p, 0), kkrest_of(u3 ? p + W : p, 0, P.kk_struct), fx, fy, fz, bad);
-            add_spring<1>(u4, Pp, B4, P.kk_struct, rest_of(u4 ? p + W + 1 : p, 2), kkrest_of(u4 ? p + W + 1 : p, 2, P.kk_struct), fx, fy, fz, bad);
-            add_spring<1>(u5, Pp, B5, P.kk_bend, rest_of(u5 ? p + 2 * W : p, 4), kkrest_of(u5 ? p + 2 * W : p, 4, P.kk_bend), fx, fy, fz, bad);
+            add_spring<1>(u0, Pp, B0, kk_struct(), rest_of(u0 ? p + 1 : p, 1), kkrest_of(u0 ? p + 1 : p, 1, kk_struct()), fx, fy, fz, bad);
+            add_spring<1>(u1, Pp, B1, kk_bend(), rest_of(u1 ? p + 2 : p, 5), kkrest_of(u1 ? p + 2 : p, 5, kk_bend()), fx, fy, fz, bad);
+            add_spring<1>(u2, Pp, B2, kk_struct(), rest_of(u2 ? p + W - 1 : p, 3), kkrest_of(u2 ? p + W - 1 : p, 3, kk_struct()), fx, fy, fz, bad);
+            add_spring<1>(u3, Pp, B3, kk_struct(), rest_of(u3 ? p + W : p, 0), kkrest_of(u3 ? p + W : p, 0, kk_struct()), fx, fy, fz, bad);
+            add_spring<1>(u4, Pp, B4, kk_struct(), rest_of(u4 ? p + W + 1 : p, 2), kkrest_of(u4 ? p + W + 1 : p, 2, kk_struct()), fx, fy, fz, bad);
+            add_spring<1>(u5, Pp, B5, kk_bend(), rest_of(u5 ? p + 2 * W : p, 4), kkrest_of(u5 ? p + 2 * W : p, 4, kk_bend()), fx, fy, fz, bad);
             // Verlet: new = x + damp*(x-px) + f*dsdm
-            T nx = Pp.x + (P.damp * (Pp.x - Q.x)) + (fx * P.dsdm);
-            T ny = Pp.y + (P.damp * (Pp.y - Q.y)) + (fy * P.dsdm);
-            T nz = Pp.z + (P.damp * (Pp.z - Q.z)) + (fz * P.dsdm);
+            T nx = Pp.x + (damp() * (Pp.x - Q.x)) + (fx * dsdm());
+            T ny = Pp.y + (damp() * (Pp.y - Q.y)) + (fy * dsdm());
+            T nz = Pp.z + (damp() * (Pp.z - Q.z)) + (fz * dsdm());
             prev[p] = mk4(nx, ny, nz, Q.w);
         }
         if (bad) misc[3] = 1;
@@ -509,7 +564,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
         T tx = Q.x + t * T(-0.0), ty = Q.y + t * T(-0.0), tz = Q.z + t * T(-1.0);
         T gx = tx + P.surf_off * T(0.0), gy = ty + P.surf_off * T(0.0), gz = tz + P.surf_off * T(1.0);
         T cx = gx - Q.x, cy = gy - Q.y, cz = gz - Q.z;
-        pos[p] = mk4(Q.x + cx * P.fric1, Q.y + cy * P.fric1, Q.z + cz * P.fric1, Pp.w);
+        pos[p] = mk4(Q.x + cx * fric1(), Q.y + cy * fric1(), Q.z + cz * fric1(), Pp.w);
     }
     // ordered replay of one bucket by one warp: from the first hit point on (nothing before it moved, so its
     // own evaluation equals the snapshot), in index order; contributions are summed in candidate order.
@@ -588,7 +643,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
                     T tx = Q.x + t * T(-0.0), ty = Q.y + t * T(-0.0), tz = Q.z + t * T(-1.0);
                     T gx = tx + P.surf_off * T(0.0), gy = ty + P.surf_off * T(0.0), gz = tz + P.surf_off * T(1.0);
                     T ex = gx - Q.x, ey = gy - Q.y, ez = gz - Q.z;
-                    Pm[k] = mk4(Q.x + ex * P.fric1, Q.y + ey * P.fric1, Q.z + ez * P.fric1, Pm[k].w);
+                    Pm[k] = mk4(Q.x + ex * fric1(), Q.y + ey * fric1(), Q.z + ez * fric1(), Pm[k].w);
                     dirty[k] = true;
                 }
                 if (dirty[k]) pos[mine[k]] = Pm[k];
@@ -850,7 +905,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
                     T tx = Q.x + t * T(-0.0), ty = Q.y + t * T(-0.0), tz = Q.z + t * T(-1.0);
                     T gx = tx + P.surf_off * T(0.0), gy = ty + P.surf_off * T(0.0), gz = tz + P.surf_off * T(1.0);
                     T ex = gx - Q.x, ey = gy - Q.y, ez = gz - Q.z;
-                    Pm = mk4(Q.x + ex * P.fric1, Q.y + ey * P.fric1, Q.z + ez * P.fric1, Pm.w);
+                    Pm = mk4(Q.x + ex * fric1(), Q.y + ey * fric1(), Q.z + ez * fric1(), Pm.w);
                     dirty = true;
                 }
                 if (dirty) pos[mine] = Pm;
@@ -912,14 +967,14 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
     // ---- _limit_spring_changes (cloth.pyx:258-296) ----
     // c_min = min(rest*1.1, rest*tear_thresh): a spring longer than that needs the sequential treatment
     __device__ __forceinline__ T limit_c(T rst) const {
-        const T a = rst * T(1.1), b = rst * P.tear_thresh;
+        const T a = rst * T(1.1), b = rst * tear_thresh();
         return a < b ? a : b;
     }
     __device__ __forceinline__ bool spring_flagged(const P4 &Pa, const P4 &Pb, T rst, int k) const {
         if (Pa.w != T(0) && Pb.w != T(0)) return false;
         if (FAST && !REST_TABLE) {       // per-kind constant: the same product limit_c() forms, squared once on the host side
             const T d0 = Pa.x - Pb.x, d1 = Pa.y - Pb.y, d2 = Pa.z - Pb.z;
-            return d0 * d0 + d1 * d1 + d2 * d2 > P.limit_c2_k[k];
+            return d0 * d0 + d1 * d1 + d2 * d2 > limit_c2_k(k);
         }
         return longer_than(Pa.x - Pb.x, Pa.y - Pb.y, Pa.z - Pb.z, limit_c(rst));
     }
@@ -1007,7 +1062,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
             if (FAST) {
                 // branch-free: the correction factor is always computed, the stores and the re-test are predicated
                 float c11, ct2;
-                if (REST_TABLE) { const float r = (float)__ldg(rest + s), ct = r * (float)P.tear_thresh; c11 = r * 1.1f; ct2 = ct * ct; }
+                if (REST_TABLE) { const float r = (float)__ldg(rest + s), ct = r * (float)tear_thresh(); c11 = r * 1.1f; ct2 = ct * ct; }
                 else { const float2 c = kc[k]; c11 = c.x; ct2 = c.y; }
                 const float e0 = (float)(Pa.x - Pb.x), e1 = (float)(Pa.y - Pb.y), e2 = (float)(Pa.z - Pb.z);
                 const float qd = e0 * e0 + e1 * e1 + e2 * e2;
@@ -1024,7 +1079,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
                 const T e0 = Pa.x - Pb.x, e1 = Pa.y - Pb.y, e2 = Pa.z - Pb.z;
                 const T c11 = rst * T(1.1);
                 const T l = norm3(e0, e1, e2);
-                if (l > rst * P.tear_thresh) misc[2] = 1;
+                if (l > rst * tear_thresh()) misc[2] = 1;
                 if (l > c11) {
                     const T d0 = e0 / l, d1 = e1 / l, d2 = e2 / l;
                     const T extra = l - c11;
@@ -1082,7 +1137,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
             P4 *pa_ptr = reinterpret_cast<P4 *>(reinterpret_cast<unsigned char *>(pos) + ao), *pb_ptr = reinterpret_cast<P4 *>(reinterpret_cast<unsigned char *>(pos) + qo);
             const P4 Pa = *pa_ptr, Pb = *pb_ptr;
             float c11, ct2;
-            if (REST_TABLE) { c11 = (float)rst_tab * 1.1f; const float ct = (float)rst_tab * (float)P.tear_thresh; ct2 = ct * ct; }
+            if (REST_TABLE) { c11 = (float)rst_tab * 1.1f; const float ct = (float)rst_tab * (float)tear_thresh(); ct2 = ct * ct; }
             else { const float2 c = kc[k]; c11 = c.x; ct2 = c.y; }
             const bool pa = Pa.w != T(0), pb = Pb.w != T(0);
             const float e0 = (float)(Pa.x - Pb.x), e1 = (float)(Pa.y - Pb.y), e2 = (float)(Pa.z - Pb.z);
@@ -1108,7 +1163,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
                 const T e0 = Pa.x - Pb.x, e1 = Pa.y - Pb.y, e2 = Pa.z - Pb.z;
                 const T c11 = rst * T(1.1);
                 const T l = norm3(e0, e1, e2);
-                if (l > rst * P.tear_thresh) misc[2] = 1;
+                if (l > rst * tear_thresh()) misc[2] = 1;
                 if (l > c11) {
                     const T d0 = e0 / l, d1 = e1 / l, d2 = e2 / l;
                     const T extra = l - c11;
@@ -1267,7 +1322,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false> st
             const T e0 = Pa.x - Pb.x, e1 = Pa.y - Pb.y, e2 = Pa.z - Pb.z;
             const T c11 = rst * T(1.1);
             const T qd = e0 * e0 + e1 * e1 + e2 * e2;
-            const T ct = rst * P.tear_thresh;
+            const T ct = rst * tear_thresh();
             if (qd > ct * ct) misc[2] = 1;
             if (qd > c11 * c11) {
                 T fac;

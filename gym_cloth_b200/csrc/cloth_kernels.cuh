@@ -12,6 +12,12 @@ extern std::atomic<long long> g_launch_count;   // defined in cloth_abi.cu
 extern int g_debug_flags;
 extern int g_force_slots, g_force_slice;         // tests: clothb200_debug_set_slicing
 extern long long *g_prof_ptr;
+// clothb200_step_kernel_info: when set, launch_step_inst reports the kernel it would launch instead of launching it
+struct KernelInfo { int ctas_per_sm, registers, local_bytes, smem_bytes; };
+extern thread_local KernelInfo *g_kernel_query;
+// cloth_abi.cu: the calling thread's buffer for per-environment material rows on the current device (see there)
+void *material_rows(size_t bytes, cudaStream_t st, int *rc);
+int material_rows_release(cudaStream_t st);
 #define CLOTHB200_MAX_DEVICES 64                    // debug: per-env phase counters (clothb200_debug_set_profile)
 void set_cuda_error(cudaError_t e, const char *where);
 
@@ -21,9 +27,10 @@ void set_cuda_error(cudaError_t e, const char *where);
 // f32, 128 threads: eight cloths per SM need <= 64 registers per thread (the shared-memory footprint allows exactly eight)
 // (f64: four per SM by shared memory -> 128 registers)
 template <typename T, int NT> struct MinBlocks { static constexpr int v = NT == 128 ? (sizeof(T) == 4 ? 8 : 4) : 1; };
-template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED>
+// PHYS: every cloth takes its material constants from its own row A.mat[env] (per-environment physics) instead of P
+template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED, bool PHYS>
 __global__ void __launch_bounds__(NT, MinBlocks<T, NT>::v) cloth_step_kernel(const __grid_constant__ DevParams<T> P, const __grid_constant__ StepArgs<T> A) {
-    typedef ClothCTA<T, NT, WC, REST_TABLE, COLOURED> CTA;
+    typedef ClothCTA<T, NT, WC, REST_TABLE, COLOURED, PHYS> CTA;
     typedef typename CTA::P4 P4;
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x;
@@ -48,7 +55,9 @@ __global__ void __launch_bounds__(NT, MinBlocks<T, NT>::v) cloth_step_kernel(con
     }
     const int env = A.env_order ? A.env_order[item] : item;
     const T *rest_env = REST_TABLE ? A.rest + (long long)env * A.rest_env_stride : nullptr;
-    CTA c(P, smem, rest_env);
+    // (a resumed cloth of the time-sliced launch comes through here again: it takes its row again)
+    const DevMaterial<T> *mat = PHYS ? A.mat + item : nullptr;
+    CTA c(P, smem, rest_env, mat);
     c.prof_on = A.prof != nullptr;
     unsigned long long gt0 = 0;
     if (A.prof && threadIdx.x == 0) { asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt0)); }
@@ -69,10 +78,12 @@ __global__ void __launch_bounds__(NT, MinBlocks<T, NT>::v) cloth_step_kernel(con
     // misc[8..11]: a pinned point at the origin that nobody writes - the idle lanes of the f32 sweep read it
     if (tid < 16) { c.misc[tid] = (tid == 11 && sizeof(T) == 4) ? 0x3f800000 : 0; c.pacc[tid] = 0; }
     if (tid < 8) {
-        const float r = (float)P.rest_k[tid < 6 ? tid : 0], ct = r * (float)P.tear_thresh;
+        const float r = (float)P.rest_k[tid < 6 ? tid : 0], ct = r * (float)c.tear_thresh();
         c.kc[tid] = make_float2(r * 1.1f, ct * ct);
     }
     int flags_in = A.flags ? A.flags[env] : 0;
+    // a material row that derive_material() rejected: the cloth is not stepped (as a CLOTHB200_PLAN_BAD_ACTION plan)
+    const bool bad_mat = PHYS ? __ldg(&mat->valid) == 0 : false;
     mbar_wait(bar, bar_phase);
     bar_phase ^= 1u;
     c.sync();
@@ -87,7 +98,7 @@ __global__ void __launch_bounds__(NT, MinBlocks<T, NT>::v) cloth_step_kernel(con
     const bool stepping = A.mode == KMODE_STEP;
     if (stepping) {
         const ClothB200Plan plan = A.plans[env];
-        const bool bad_action = (plan.reserved & CLOTHB200_PLAN_BAD_ACTION) != 0;   // NaN action: nothing is gripped, BADSTATE
+        const bool bad_action = (plan.reserved & CLOTHB200_PLAN_BAD_ACTION) != 0 || bad_mat;   // NaN action: nothing is gripped, BADSTATE
         if (bad_action) { ngrab = 0; if (tid == 0) c.misc[3] = 1; }
         else if (i_begin > 0) ngrab = ngrab_in;       // resumed slice: the grip is part of the stored state
         else ngrab = c.grab_top(plan.gx, plan.gy, P.grip_radius);
@@ -106,7 +117,8 @@ __global__ void __launch_bounds__(NT, MinBlocks<T, NT>::v) cloth_step_kernel(con
         iterations = ngrab == 0 ? 0 : (int)ceil(t4);   // cloth_env.py:490-493
         dxr = (T)plan.dxr; dyr = (T)plan.dyr;
     } else if (A.mode == KMODE_UPDATE) {
-        iterations = A.n_updates;
+        iterations = bad_mat ? 0 : A.n_updates;
+        if (bad_mat && tid == 0) c.misc[3] = 1;
     } else if (A.mode == KMODE_GRAB) {
         ngrab = c.grab_top(A.grab_xy[2 * env], A.grab_xy[2 * env + 1], A.grab_radius);
         if (A.grab_mask) c.write_grab_mask(A.grab_mask + (size_t)env * ((N + 31) >> 5));
@@ -403,14 +415,6 @@ template <typename T> int make_dev_params(const ClothB200Params &hp, DevParams<T
     P.table_shift = 32 - sh;
     P.ev_words = (6 * P.N + 31) / 32;
     P.max_actions = hp.max_actions;
-    // constants exactly as cloth.pyx:175-186, 240-241 derive them, in double, then rounded to T once
-    const double mass = hp.density / W / H;
-    const double delta_t = 1.0 / hp.frames_per_sec / hp.simulation_steps;
-    P.mg = (T)(mass * hp.gravity);
-    P.kk_struct = (T)(hp.ks * 1.0);
-    P.kk_bend = (T)(hp.ks * 0.2);
-    P.dsdm = (T)((delta_t * delta_t) / mass);
-    P.damp = (T)(1.0 - hp.damping / 100.0);
     const double dx = hp.width * 1.0 / (W - 1), dy = hp.height * 1.0 / (H - 1);
     const double cw = 3 * dx, ch = 3 * dy;
     P.cell_w = (T)cw; P.cell_h = (T)ch; P.cell_t = (T)(cw > ch ? cw : ch);
@@ -424,17 +428,17 @@ template <typename T> int make_dev_params(const ClothB200Params &hp, DevParams<T
     }
     P.sim_steps = (T)hp.simulation_steps;
     P.min_z = (T)hp.minimum_z;
-    P.fric1 = (T)(1. - hp.plane_friction);
     P.surf_off = (T)0.0001;
-    P.tear_thresh = (T)hp.tear_thresh;
     const double diag = sqrt(dx * dx + dy * dy);
     const double rk[6] = {dx, dy, diag, diag, 2 * dx, 2 * dy};
-    for (int k = 0; k < 6; k++) {
-        P.rest_k[k] = (T)rk[k];
-        P.kkrest_k[k] = (k >= 4 ? P.kk_bend : P.kk_struct) * P.rest_k[k];
-        const T a = P.rest_k[k] * T(1.1), b = P.rest_k[k] * P.tear_thresh, c = a < b ? a : b;    // ClothCTA::limit_c
-        P.limit_c2_k[k] = c * c;
-    }
+    for (int k = 0; k < 6; k++) P.rest_k[k] = (T)rk[k];
+    // the material constants (mass*gravity, ks terms, damping, friction, tear threshold)
+    DevMaterial<T> m;
+    derive_material<T>(hp.density, hp.ks, hp.damping, hp.plane_friction, hp.tear_thresh, hp.gravity, W, H, hp.frames_per_sec,
+                       hp.simulation_steps, P.rest_k, m);
+    P.mg = m.mg; P.kk_struct = m.kk_struct; P.kk_bend = m.kk_bend; P.dsdm = m.dsdm; P.damp = m.damp;
+    P.fric1 = m.fric1; P.tear_thresh = m.tear_thresh;
+    for (int k = 0; k < 6; k++) { P.kkrest_k[k] = m.kkrest_k[k]; P.limit_c2_k[k] = m.limit_c2_k[k]; }
     P.grip_radius = hp.grip_radius; P.thickness = hp.thickness; P.gripper_height = hp.gripper_height;
     int nlev = 0;
     for (double z = hp.gripper_height; z > 0; z -= hp.thickness) { nlev++; if (nlev > 8 * ts / 8) break; }
@@ -448,10 +452,10 @@ template <typename T> int make_dev_params(const ClothB200Params &hp, DevParams<T
     return 0;
 }
 
-template <typename T, int NT, int WC, bool RT, bool COL> int launch_step_inst(const DevParams<T> &P, const StepArgs<T> &A, cudaStream_t st) {
-    typedef ClothCTA<T, NT, WC, RT, COL> CTA;
+template <typename T, int NT, int WC, bool RT, bool COL, bool PHYS> int launch_step_inst(const DevParams<T> &P, const StepArgs<T> &A, cudaStream_t st) {
+    typedef ClothCTA<T, NT, WC, RT, COL, PHYS> CTA;
     const size_t smem = CTA::smem_bytes(P.N, P.table_size, P.ev_words);
-    auto kern = cloth_step_kernel<T, NT, WC, RT, COL>;
+    auto kern = cloth_step_kernel<T, NT, WC, RT, COL, PHYS>;
     // cudaFuncSetAttribute and occupancy are per device: one process may drive several GPUs (SURVEY.md 8(e) allows one
     // process with a stream per device), so both caches are keyed by the current device
     static std::atomic<size_t> configured[CLOTHB200_MAX_DEVICES];
@@ -469,6 +473,16 @@ template <typename T, int NT, int WC, bool RT, bool COL> int launch_step_inst(co
             return CLOTHB200_ERR_UNSUPPORTED;
         }
         configured[dev].store(smem);
+    }
+    if (g_kernel_query) {
+        cudaFuncAttributes fa;
+        int occ = 0;
+        if (cudaFuncGetAttributes(&fa, kern) != cudaSuccess || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem) != cudaSuccess) {
+            set_cuda_error(cudaGetLastError(), "step kernel attributes");
+            return CLOTHB200_ERR_CUDA;
+        }
+        *g_kernel_query = KernelInfo{occ, fa.numRegs, (int)fa.localSizeBytes, (int)smem};
+        return CLOTHB200_OK;
     }
     if (A.slice > 0) {
         // time-sliced mode: a persistent grid, one CTA per resident slot; pointless when every cloth has its own slot
@@ -507,36 +521,57 @@ int endgame_slices();           // cloth_abi.cu: CLOTHB200_ENDGAME env var (slic
 int endgame_shift();
 int threads_per_cloth(int W);   // cloth_abi.cu: CLOTHB200_NT env var; default 128 (512 for 64x64)
 
-template <typename T, int WC, bool RT, bool COL> int launch_step_nt(const DevParams<T> &P, const StepArgs<T> &A, cudaStream_t st) {
+template <typename T, int WC, bool RT, bool COL, bool PHYS> int launch_step_nt(const DevParams<T> &P, const StepArgs<T> &A, cudaStream_t st) {
     const int nt = threads_per_cloth(P.W);
     if (WC == 64) {   // one resident cloth per SM: wide CTAs
-        if (nt == 256) return launch_step_inst<T, 256, WC, RT, COL>(P, A, st);
-        return launch_step_inst<T, 512, WC, RT, COL>(P, A, st);
+        if (nt == 256) return launch_step_inst<T, 256, WC, RT, COL, PHYS>(P, A, st);
+        return launch_step_inst<T, 512, WC, RT, COL, PHYS>(P, A, st);
     }
-    if (nt == 256) return launch_step_inst<T, 256, WC, RT, COL>(P, A, st);
-    return launch_step_inst<T, 128, WC, RT, COL>(P, A, st);
+    if (nt == 256) return launch_step_inst<T, 256, WC, RT, COL, PHYS>(P, A, st);
+    return launch_step_inst<T, 128, WC, RT, COL, PHYS>(P, A, st);
 }
 
-// One (scalar type, compile-time grid width) pair per translation unit (cloth_inst.cu, built six times in
-// parallel): the kernel is one large force-inlined function and a single TU holding every variant compiles for
-// a quarter of an hour.
-template <typename T, int WC> int launch_step_wc(const DevParams<T> &P, const StepArgs<T> &A, cudaStream_t st, bool rt, bool coloured) {
+// One (scalar type, compile-time grid width, per-environment material or not) triple per translation unit
+// (cloth_inst.cu, built twelve times in parallel): the kernel is one large force-inlined function and a single TU
+// holding every variant compiles for a quarter of an hour.
+template <typename T, int WC, bool PHYS> int launch_step_wc(const DevParams<T> &P, const StepArgs<T> &A, cudaStream_t st, bool rt, bool coloured) {
     if (coloured) {
-        if constexpr (WC != 0) return rt ? launch_step_nt<T, WC, true, true>(P, A, st) : launch_step_nt<T, WC, false, true>(P, A, st);
+        if constexpr (WC != 0) return rt ? launch_step_nt<T, WC, true, true, PHYS>(P, A, st) : launch_step_nt<T, WC, false, true, PHYS>(P, A, st);
         else return CLOTHB200_ERR_UNSUPPORTED;   // coloured mode is built for the 25x25 and 64x64 grids
     }
-    return rt ? launch_step_nt<T, WC, true, false>(P, A, st) : launch_step_nt<T, WC, false, false>(P, A, st);
+    return rt ? launch_step_nt<T, WC, true, false, PHYS>(P, A, st) : launch_step_nt<T, WC, false, false, PHYS>(P, A, st);
 }
 #ifdef CLOTH_INSTANTIATE_WC
-template int launch_step_wc<CLOTH_T, CLOTH_INSTANTIATE_WC>(const DevParams<CLOTH_T> &, const StepArgs<CLOTH_T> &, cudaStream_t, bool, bool);
+#ifndef CLOTH_INSTANTIATE_PHYS
+#define CLOTH_INSTANTIATE_PHYS 0
+#endif
+template int launch_step_wc<CLOTH_T, CLOTH_INSTANTIATE_WC, CLOTH_INSTANTIATE_PHYS != 0>(const DevParams<CLOTH_T> &, const StepArgs<CLOTH_T> &, cudaStream_t, bool, bool);
 #else
-#define CLOTH_EXTERN_WC(T, WC) extern template int launch_step_wc<T, WC>(const DevParams<T> &, const StepArgs<T> &, cudaStream_t, bool, bool);
-CLOTH_EXTERN_WC(float, 0) CLOTH_EXTERN_WC(float, 25) CLOTH_EXTERN_WC(float, 64)
-CLOTH_EXTERN_WC(double, 0) CLOTH_EXTERN_WC(double, 25) CLOTH_EXTERN_WC(double, 64)
+#define CLOTH_EXTERN_WC(T, WC, PH) extern template int launch_step_wc<T, WC, PH>(const DevParams<T> &, const StepArgs<T> &, cudaStream_t, bool, bool);
+CLOTH_EXTERN_WC(float, 0, false) CLOTH_EXTERN_WC(float, 25, false) CLOTH_EXTERN_WC(float, 64, false)
+CLOTH_EXTERN_WC(double, 0, false) CLOTH_EXTERN_WC(double, 25, false) CLOTH_EXTERN_WC(double, 64, false)
+CLOTH_EXTERN_WC(float, 0, true) CLOTH_EXTERN_WC(float, 25, true) CLOTH_EXTERN_WC(float, 64, true)
+CLOTH_EXTERN_WC(double, 0, true) CLOTH_EXTERN_WC(double, 25, true) CLOTH_EXTERN_WC(double, 64, true)
 #undef CLOTH_EXTERN_WC
 #endif
 
-template <typename T> int launch_step(const ClothB200Params &hp, const StepArgs<T> &A, cudaStream_t st, int rmode = 0) {
+// per-environment material rows, by launch position i (the step kernel's `item`): row i holds the constants of
+// environment env_order[i] (or i), derived by the same derive_material() make_dev_params calls
+template <typename T>
+__global__ void derive_material_kernel(int n, const ClothB200Physics *__restrict__ phys, const int32_t *__restrict__ env_order,
+                                       const __grid_constant__ DevParams<T> P, double frames_per_sec, int simulation_steps,
+                                       DevMaterial<T> *__restrict__ mat) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const ClothB200Physics ph = phys[env_order ? env_order[i] : i];
+    DevMaterial<T> m;
+    derive_material<T>(ph.density, ph.ks, ph.damping, ph.plane_friction, ph.tear_thresh, ph.gravity, P.W, P.H, frames_per_sec,
+                       simulation_steps, P.rest_k, m);
+    mat[i] = m;
+}
+
+template <typename T>
+int launch_step(const ClothB200Params &hp, const StepArgs<T> &A, cudaStream_t st, int rmode = 0, const ClothB200Physics *phys = nullptr) {
     if (A.n_env == 0) return CLOTHB200_OK;
     DevParams<T> P;
     make_dev_params(hp, P);
@@ -544,9 +579,35 @@ template <typename T> int launch_step(const ClothB200Params &hp, const StepArgs<
     const bool rt = A.rest != nullptr;
     if (!rt && sizeof(T) == 8 && rmode == 0) return CLOTHB200_ERR_ARG;  // the parity build always takes the exact rest table
     const bool coloured = rmode == CLOTHB200_MODE_COLOURED;
-    if (P.W == 25 && P.H == 25) return launch_step_wc<T, 25>(P, A, st, rt, coloured);
-    if (P.W == 64 && P.H == 64) return launch_step_wc<T, 64>(P, A, st, rt, coloured);
-    return launch_step_wc<T, 0>(P, A, st, rt, coloured);
+    if (phys) {
+        StepArgs<T> B = A;
+        int rc = CLOTHB200_OK;
+        if (!g_kernel_query) {
+            // the rows go to the calling thread's cached buffer (no allocation per call); it is released to the next call
+            // behind this call's step kernel
+            DevMaterial<T> *mat = (DevMaterial<T> *)material_rows(sizeof(DevMaterial<T>) * (size_t)A.n_env, st, &rc);
+            if (rc) return rc;
+            derive_material_kernel<T><<<(A.n_env + 127) / 128, 128, 0, st>>>(A.n_env, phys, A.env_order, P, (double)hp.frames_per_sec,
+                                                                             hp.simulation_steps, mat);
+            g_launch_count++;
+            const cudaError_t e = cudaGetLastError();
+            if (e != cudaSuccess) { set_cuda_error(e, "derive_material_kernel"); rc = CLOTHB200_ERR_CUDA; }
+            B.mat = mat;
+        }
+        if (rc == CLOTHB200_OK) {
+            if (P.W == 25 && P.H == 25) rc = launch_step_wc<T, 25, true>(P, B, st, rt, coloured);
+            else if (P.W == 64 && P.H == 64) rc = launch_step_wc<T, 64, true>(P, B, st, rt, coloured);
+            else rc = launch_step_wc<T, 0, true>(P, B, st, rt, coloured);
+        }
+        if (!g_kernel_query) {
+            const int rc2 = material_rows_release(st);
+            if (rc == CLOTHB200_OK) rc = rc2;
+        }
+        return rc;
+    }
+    if (P.W == 25 && P.H == 25) return launch_step_wc<T, 25, false>(P, A, st, rt, coloured);
+    if (P.W == 64 && P.H == 64) return launch_step_wc<T, 64, false>(P, A, st, rt, coloured);
+    return launch_step_wc<T, 0, false>(P, A, st, rt, coloured);
 }
 
 template <typename T> size_t step_smem_bytes(const ClothB200Params &hp) {

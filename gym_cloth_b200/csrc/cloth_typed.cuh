@@ -36,7 +36,7 @@ template <typename T> int check_io(int n_env, const ClothB200Step *io) {
 
 template <typename T>
 int step_plans_t(const ClothB200Params *hp, int mode, int n_env, const ClothB200Plan *plans, const ClothB200Step *io, int initialize,
-                 cudaStream_t st) {
+                 const ClothB200Physics *phys, cudaStream_t st) {
     int rc = check_io<T>(n_env, io);
     if (rc || n_env == 0) return rc;
     if (!hp || !plans) return CLOTHB200_ERR_ARG;
@@ -71,18 +71,19 @@ int step_plans_t(const ClothB200Params *hp, int mode, int n_env, const ClothB200
             A.slice = slice; A.yield_slack = yield_slack_substeps(); A.endgame_slices = endgame_slices(); A.endgame_shift = endgame_shift(); A.qcap = n_env; A.sorted_keys = keys;
         }
     }
-    return launch_step<T>(*hp, A, st, mode);
+    return launch_step<T>(*hp, A, st, mode, phys);
 }
 
 template <typename T>
-int update_n_t(const ClothB200Params *hp, int mode, int n_env, int n_updates, const ClothB200Step *io, cudaStream_t st) {
+int update_n_t(const ClothB200Params *hp, int mode, int n_env, int n_updates, const ClothB200Step *io, const ClothB200Physics *phys,
+               cudaStream_t st) {
     int rc = check_io<T>(n_env, io);
     if (rc || n_env == 0) return rc;
     if (!hp || n_updates < 0) return CLOTHB200_ERR_ARG;
     if (mode != CLOTHB200_MODE_REFERENCE_ORDER && mode != CLOTHB200_MODE_COLOURED) return CLOTHB200_ERR_UNSUPPORTED;
     StepArgs<T> A = make_args<T>(n_env, io);
     A.mode = KMODE_UPDATE; A.n_updates = n_updates;
-    return launch_step<T>(*hp, A, st, mode);
+    return launch_step<T>(*hp, A, st, mode, phys);
 }
 
 template <typename T>
@@ -93,6 +94,21 @@ int grab_top_t(const ClothB200Params *hp, int n_env, const double *xy, double ra
     StepArgs<T> A = make_args<T>(n_env, io);
     A.mode = KMODE_GRAB; A.grab_xy = xy; A.grab_radius = radius;
     return launch_step<T>(*hp, A, st);
+}
+
+// the step kernel that step_plans would launch for this configuration, queried instead of launched
+template <typename T> int kernel_info_t(const ClothB200Params *hp, int mode, int rest_table, int per_env_physics, int *out) {
+    StepArgs<T> A = make_args<T>(1, nullptr);
+    A.mode = KMODE_STEP;
+    static const T dummy_rest[1] = {T(0)};
+    A.rest = rest_table ? dummy_rest : nullptr;              // only tested for NULL: nothing is read
+    static const ClothB200Physics dummy_phys = {};
+    KernelInfo info = {0, 0, 0, 0};
+    g_kernel_query = &info;
+    const int rc = launch_step<T>(*hp, A, 0, mode, per_env_physics ? &dummy_phys : nullptr);
+    g_kernel_query = nullptr;
+    out[0] = info.ctas_per_sm; out[1] = info.registers; out[2] = info.local_bytes; out[3] = info.smem_bytes;
+    return rc;
 }
 
 template <typename T> int measure_t(const ClothB200Params *hp, int n_env, const ClothB200Step *io, cudaStream_t st) {

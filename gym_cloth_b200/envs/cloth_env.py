@@ -78,7 +78,7 @@ class BatchedClothEnv(object):
     """
 
     def __init__(self, cfg, n_env, dtype="f32", device=None, seed=None, env_offset=0, dom_rand_draws=False,
-                 mode=_l.MODE_REFERENCE_ORDER):
+                 mode=_l.MODE_REFERENCE_ORDER, physics=None):
         self.cfg = load_cfg(cfg)
         cfg = self.cfg
         self.P = _l.params_from_cfg(cfg)
@@ -126,7 +126,42 @@ class BatchedClothEnv(object):
         self.start_coverage = torch.zeros(self.n_env, dtype=torch.float64, device=self.device)
         self.start_variance_inv = torch.zeros(self.n_env, dtype=torch.float64, device=self.device)
         self._pinned = None
+        if physics is not None:
+            self.set_physics(**physics)
         self.seed(cfg.get("seed", 0) if seed is None else seed)
+
+    # ------------------------------------------------------------------ per-environment material
+    def get_physics(self):
+        """The material of every environment: dict of float64 arrays [n_env] (lib.PHYSICS_FIELDS)."""
+        if self.cloth.physics is None:
+            return {k: np.full(self.n_env, float(getattr(self.P, k))) for k in _l.PHYSICS_FIELDS}
+        t = self.cloth.physics.cpu().numpy()
+        return {k: t[:, i].copy() for i, k in enumerate(_l.PHYSICS_FIELDS)}
+
+    def set_physics(self, envs=None, density=None, ks=None, damping=None, plane_friction=None, tear_thresh=None, gravity=None):
+        """Give the selected environments (all by default) their own material: each value a scalar or one value per
+        selected environment; a field left None keeps its current value (initially the cfg's).  The values persist
+        across reset(), whose pulls and settle loops run under each environment's own material.  Raises ValueError for
+        a wrong length, a non-finite value or density <= 0."""
+        sel = self._sel(envs)
+        if len(sel) and (sel.min() < 0 or sel.max() >= self.n_env):
+            raise ValueError("environment index out of range")
+        given = {k: v for k, v in (("density", density), ("ks", ks), ("damping", damping), ("plane_friction", plane_friction),
+                                   ("tear_thresh", tear_thresh), ("gravity", gravity)) if v is not None}
+        new = {}
+        for k, v in given.items():
+            a = np.asarray(v, np.float64)
+            if a.ndim == 0:
+                a = np.full(len(sel), float(a))
+            if a.shape != (len(sel),):
+                raise ValueError("%s: expected a scalar or %d values, got shape %s" % (k, len(sel), a.shape))
+            if not np.all(np.isfinite(a)):
+                raise ValueError("%s: values must be finite" % k)
+            if k == "density" and not np.all(a > 0):
+                raise ValueError("density must be > 0")
+            new[k] = a
+        if new:
+            self.cloth.set_physics(envs=sel, **new)
 
     # ------------------------------------------------------------------ seeding
     def seed(self, seed=None):

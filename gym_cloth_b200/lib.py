@@ -63,6 +63,16 @@ class Step(C.Structure):
     ]
 
 
+class Physics(C.Structure):
+    """ClothB200Physics: one environment's material (the `_phys` entry points take a device array of these)."""
+    _fields_ = [("density", C.c_double), ("ks", C.c_double), ("damping", C.c_double), ("plane_friction", C.c_double),
+                ("tear_thresh", C.c_double), ("gravity", C.c_double), ("reserved", C.c_double * 2)]
+
+
+# the fields of a ClothB200Physics row, in order (a [n_env, 8] float64 tensor holds them and two zero columns)
+PHYSICS_FIELDS = ("density", "ks", "damping", "plane_friction", "tear_thresh", "gravity")
+
+
 class Scene(C.Structure):
     """ClothB200Scene: the Blender scene of gym_cloth/blender/get_image_rep_279.py."""
     _f3 = C.c_float * 3
@@ -94,8 +104,10 @@ _PROTOS = {
     "clothb200_sizeof_params": (C.c_size_t, []),
     "clothb200_sizeof_plan": (C.c_size_t, []),
     "clothb200_sizeof_step": (C.c_size_t, []),
+    "clothb200_sizeof_physics": (C.c_size_t, []),
     "clothb200_device_info": (_i, [_i] + [C.POINTER(C.c_int)] * 4),
     "clothb200_occupancy": (_i, [_PP, _i] + [C.POINTER(C.c_int)] * 3),
+    "clothb200_step_kernel_info": (_i, [_PP, _i, _i, _i, _i] + [C.POINTER(C.c_int)] * 4),
     "clothb200_params_default": (_i, [_PP]),
     "clothb200_params_validate": (_i, [_PP]),
     "clothb200_decode_actions_host": (_i, [_PP, _i, _vp, _vp]),
@@ -122,6 +134,10 @@ _TYPED = {
     "clothb200_gripper_release": (_i, [_i, _i, _vp, _vp, _vp]),
     "clothb200_measure": (_i, [_PP, _i, _SP, _vp]),
     "clothb200_step_host": (_i, [_PP, _i, _i, _vp, _SP, _i] + [_vp] * 8),
+    "clothb200_step_plans_phys": (_i, [_PP, _i, _i, _vp, _SP, _i, _vp, _vp]),
+    "clothb200_step_actions_phys": (_i, [_PP, _i, _i, _vp, _vp, _SP, _i, _vp, _vp]),
+    "clothb200_update_n_phys": (_i, [_PP, _i, _i, _i, _SP, _vp, _vp]),
+    "clothb200_step_host_phys": (_i, [_PP, _i, _i, _vp, _SP, _i] + [_vp] * 9),
     "clothb200_render_rgb": (_i, [_PP, _ScP, _SeP, _i, _vp, _vp, _vp]),
     "clothb200_render_depth": (_i, [_PP, _ScP, _SeP, _i, _vp, _vp, _vp, _vp, _vp]),
 }
@@ -163,6 +179,7 @@ def lib(variant=None):
     assert L.clothb200_sizeof_plan() == C.sizeof(Plan), "Plan layout mismatch"
     assert L.clothb200_sizeof_step() == C.sizeof(Step), "Step layout mismatch"
     assert L.clothb200_sizeof_scene() == C.sizeof(Scene), "Scene layout mismatch"
+    assert L.clothb200_sizeof_physics() == C.sizeof(Physics), "Physics layout mismatch"
     if variant is None:
         _lib = L
     else:
@@ -222,6 +239,11 @@ def params_from_cfg(cfg):
     P.reward_type = REWARD_TYPE[rt]
     check(lib().clothb200_params_validate(C.byref(P)), "params_validate")
     return P
+
+
+def physics_of(P):
+    """The material of ClothB200Params P as a dict of the ClothB200Physics fields."""
+    return {k: float(getattr(P, k)) for k in PHYSICS_FIELDS}
 
 
 def copy_params(P):

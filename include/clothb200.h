@@ -11,8 +11,8 @@
  *
  * Conventions
  *  - plain C types only; every pointer documented as HOST or DEVICE; the library never owns
- *    persistent device memory (PyTorch tensors do) except a small per-thread scratch cache
- *    used by the *_host convenience entry points.
+ *    persistent device memory (PyTorch tensors do) except small per-thread scratch caches
+ *    used by the *_host convenience entry points and for the derived rows of the *_phys_* ones.
  *  - `stream` is a cudaStream_t passed as void* (NULL = default stream).  Device entry points are
  *    asynchronous on that stream; *_host entry points synchronise the stream before returning.
  *  - return value: 0 = CLOTHB200_OK, negative = error (clothb200_error_string()).  No exceptions
@@ -142,6 +142,12 @@ size_t clothb200_sizeof_step(void);
 int clothb200_device_info(int device, int *sm_count, int *cc_major, int *cc_minor, int *smem_per_sm);
 /* resident cloths per SM / shared memory per cloth for this grid size, f32 (is_f64=0) or f64. */
 int clothb200_occupancy(const ClothB200Params *params, int is_f64, int *ctas_per_sm, int *smem_bytes, int *threads);
+/* the step kernel step_plans would launch for this grid, mode, rest-table choice (rest_table != 0: ClothB200Step.rest
+ * given) and material (per_env_physics != 0: the `_phys` entry points) on the current device, as the runtime reports
+ * it: resident CTAs per SM (cudaOccupancyMaxActiveBlocksPerMultiprocessor), registers per thread, local memory
+ * (spill) bytes per thread and dynamic shared memory per CTA.  Nothing is launched. */
+int clothb200_step_kernel_info(const ClothB200Params *params, int is_f64, int mode, int rest_table, int per_env_physics,
+                               int *ctas_per_sm, int *registers, int *local_bytes, int *smem_bytes);
 
 /* values of cfg/t1_rgbd.yaml (identical in t2/t3 apart from init.type). */
 int clothb200_params_default(ClothB200Params *params);
@@ -187,6 +193,43 @@ int clothb200_step_actions_f64(const ClothB200Params *params, int mode, int n_en
  * (cloth_env.py:902-903, 948-949, 980-981) and a bare `cloth.update()` of the facade. */
 int clothb200_update_n_f32(const ClothB200Params *params, int mode, int n_env, int n_updates, const ClothB200Step *io, void *stream);
 int clothb200_update_n_f64(const ClothB200Params *params, int mode, int n_env, int n_updates, const ClothB200Step *io, void *stream);
+
+/* ---- per-environment material (domain randomisation of the physics) ----
+ * The six cfg values Cloth.update turns into constants (cloth.pyx:53-56, 175-186, 240-241), one row per environment.
+ * The `_phys` twins below take `physics`, a DEVICE array [n_env] indexed by environment index (the index of `pos`, not
+ * the launch position: env_order subsets and the built-in longest-first order work unchanged).  Each row's constants
+ * are derived in double and rounded once, exactly as from ClothB200Params, so a row equal to the batch's values gives
+ * the plain entry point's bits.  physics == NULL is the plain entry point.  A row with a non-finite value or
+ * density <= 0 is invalid: that environment is treated like a CLOTHB200_PLAN_BAD_ACTION plan (no substep, state kept,
+ * CLOTHB200_FLAG_BADSTATE | CLOTHB200_FLAG_NOGRAB; update_n: no update, BADSTATE).  The other fields of
+ * ClothB200Params (grid, thickness, schedule, gripper) stay per batch. */
+typedef struct ClothB200Physics {
+    double density, ks, damping, plane_friction, tear_thresh, gravity;
+    double reserved[2];        /* 0 */
+} ClothB200Physics;            /* 64 bytes */
+size_t clothb200_sizeof_physics(void);
+int clothb200_step_plans_phys_f32(const ClothB200Params *params, int mode, int n_env, const ClothB200Plan *plans,
+                                  const ClothB200Step *io, int initialize, const ClothB200Physics *physics, void *stream);
+int clothb200_step_plans_phys_f64(const ClothB200Params *params, int mode, int n_env, const ClothB200Plan *plans,
+                                  const ClothB200Step *io, int initialize, const ClothB200Physics *physics, void *stream);
+int clothb200_step_actions_phys_f32(const ClothB200Params *params, int mode, int n_env, const float *actions,
+                                    ClothB200Plan *plans_scratch, const ClothB200Step *io, int initialize,
+                                    const ClothB200Physics *physics, void *stream);
+int clothb200_step_actions_phys_f64(const ClothB200Params *params, int mode, int n_env, const double *actions,
+                                    ClothB200Plan *plans_scratch, const ClothB200Step *io, int initialize,
+                                    const ClothB200Physics *physics, void *stream);
+int clothb200_update_n_phys_f32(const ClothB200Params *params, int mode, int n_env, int n_updates, const ClothB200Step *io,
+                                const ClothB200Physics *physics, void *stream);
+int clothb200_update_n_phys_f64(const ClothB200Params *params, int mode, int n_env, int n_updates, const ClothB200Step *io,
+                                const ClothB200Physics *physics, void *stream);
+int clothb200_step_host_phys_f32(const ClothB200Params *params, int mode, int n_env, const double *actions,
+                                 const ClothB200Step *io, int initialize, float *obs, double *reward, int32_t *done,
+                                 double *coverage, double *variance_inv, int32_t *flags, int32_t *sim_steps,
+                                 const ClothB200Physics *physics, void *stream);
+int clothb200_step_host_phys_f64(const ClothB200Params *params, int mode, int n_env, const double *actions,
+                                 const ClothB200Step *io, int initialize, double *obs, double *reward, int32_t *done,
+                                 double *coverage, double *variance_inv, int32_t *flags, int32_t *sim_steps,
+                                 const ClothB200Physics *physics, void *stream);
 
 /* ---- pieces, for the facade and the parity tests ---- */
 /* Gripper.grab_top(x, y) (gripper.pyx:23-42); xy DEVICE [n_env][2] doubles; grip_radius as Gripper.grip_radius. */
