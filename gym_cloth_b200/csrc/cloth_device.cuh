@@ -42,6 +42,14 @@ __device__ __forceinline__ double floor_t(double x) { return floor(x); }
 // cloth.pyx:17-18 fastnorm: sqrt(x*x + y*y + z*z), left-to-right
 template <typename T> __device__ __forceinline__ T norm3(T x, T y, T z) { return sqrt_t(x * x + y * y + z * z); }
 
+// The reward terms and the grip test in double, one rounding per operator as in the oracle (-ffp-contract=off): the
+// f32 units allow FMA contraction, which would also fuse these double products and sums; ptxas never fuses the _rn
+// intrinsics.  (-fmad=false makes the f64 units round every operator anyway: there these compile as before.)
+// dx*dx + dy*dy
+__device__ __forceinline__ double dist2_rn(double dx, double dy) { return __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)); }
+// ax*by - ay*bx: the monotone chain's turn test and the shoelace term
+__device__ __forceinline__ double cross_rn(double ax, double ay, double bx, double by) { return __dsub_rn(__dmul_rn(ax, by), __dmul_rn(ay, bx)); }
+
 template <typename T> struct DevParams {
     int W, H, N;
     int table_size, table_shift; // hash table: power of two >= 1.6 N
@@ -1400,7 +1408,8 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
             }
         }
     }
-    // grab_top (gripper.pyx:23-42) in double.  Returns len(grabbed_pts) afterwards (all threads).
+    // grab_top (gripper.pyx:23-42) in double, the radius test rounded as the oracle's (dist2_rn): both builds grip the
+    // oracle's set on their own state.  Returns len(grabbed_pts) afterwards (all threads).
     // scratch: doubles in the (idle) hash table area.
     __device__ __forceinline__ int grab_top(double x, double y, double radius) {
         double *levels = reinterpret_cast<double *>(tkey);
@@ -1416,7 +1425,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
         for (int p = tid; p < N; p += NT) {
             const P4 Pp = pos[p];
             const double px = (double)Pp.x, py = (double)Pp.y, pz = (double)Pp.z;
-            if ((px - x) * (px - x) + (py - y) * (py - y) < radius) {
+            if (dist2_rn(px - x, py - y) < radius) {
                 for (int i = 0; i < nlev && i < mylev_min; i++)
                     if (fabs(pz - levels[i]) < band) { mylev_min = i; break; }
             }
@@ -1431,7 +1440,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
             bool sel = false;
             if (lev != 0x7fffffff) {
                 const double px = (double)Pp.x, py = (double)Pp.y, pz = (double)Pp.z;
-                sel = ((px - x) * (px - x) + (py - y) * (py - y) < radius) && (fabs(pz - levels[lev]) < band);
+                sel = (dist2_rn(px - x, py - y) < radius) && (fabs(pz - levels[lev]) < band);
             }
             if (sel) {
                 Pp.w = T(1); Q.w = Q.w + T(1);
@@ -1474,11 +1483,15 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
         clipped_xy(a, ax, ay); clipped_xy(b, bx, by);
         return (ax < bx) || (ax == bx && ay < by);
     }
-    // Andrew monotone chain + shoelace in double, same operation order as oracle_hull_area.
+    // Andrew monotone chain + shoelace in double, same operations in the same order as oracle_hull_area, each rounded
+    // once (cross_rn) in both builds: the f32 build's coverage is the oracle's of its own (widened) state, bit for bit.
     // Uses the hash table area as scratch (the table is rebuilt from scratch every substep).
     __device__ __forceinline__ double hull_area() {
         uint16_t *idx = reinterpret_cast<uint16_t *>(tkey);   // [np2] spans tkey+tinfo (8*table_size bytes, table_size >= np2/4)
-        uint16_t *hull = lstA;                                // [2N] spans lstA+lstB (contiguous, idle outside update())
+        // [< 2N] from lstA on, over cls and lstB (contiguous, idle outside update()).  Points in convex position fill
+        // N + 1 entries, one more than lstA holds when N % 8 == 0: the last lands at the head of cls (or of lstB where
+        // cls aliases it), which every substep rewrites before it reads it.
+        uint16_t *hull = lstA;
         int np2 = 1; while (np2 < N) np2 <<= 1;
         for (int i = tid; i < np2; i += NT) idx[i] = (uint16_t)i;
         sync();
@@ -1503,7 +1516,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
                 clipped_xy(idx[i], bx, by);
                 while (kk >= 2) {
                     clipped_xy(hull[kk - 2], ox, oy); clipped_xy(hull[kk - 1], ax, ay);
-                    if ((ax - ox) * (by - oy) - (ay - oy) * (bx - ox) <= 0) kk--; else break;
+                    if (cross_rn(ax - ox, ay - oy, bx - ox, by - oy) <= 0) kk--; else break;
                 }
                 hull[kk++] = idx[i];
             }
@@ -1511,7 +1524,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
                 clipped_xy(idx[i], bx, by);
                 while (kk >= t) {
                     clipped_xy(hull[kk - 2], ox, oy); clipped_xy(hull[kk - 1], ax, ay);
-                    if ((ax - ox) * (by - oy) - (ay - oy) * (bx - ox) <= 0) kk--; else break;
+                    if (cross_rn(ax - ox, ay - oy, bx - ox, by - oy) <= 0) kk--; else break;
                 }
                 hull[kk++] = idx[i];
             }
@@ -1521,7 +1534,7 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
             for (int i = 0; i < kk; i++) {
                 clipped_xy(hull[i], ax, ay);
                 clipped_xy(hull[(i + 1) % kk], bx, by);
-                a2 += (ax - hx) * (by - hy) - (bx - hx) * (ay - hy);
+                a2 = __dadd_rn(a2, cross_rn(ax - hx, ay - hy, bx - hx, by - hy));
             }
             area = (kk >= 3) ? 0.5 * fabs(a2) : 0.0;
         }
@@ -1546,13 +1559,13 @@ template <typename T, int NT, int WC, bool REST_TABLE, bool COLOURED = false, bo
         sync();
         return s;
     }
-    // _compute_variance (cloth_env.py:1075-1084)
+    // _compute_variance (cloth_env.py:1075-1084): per-thread strided sums, block_sum's order, one rounding per operator
     __device__ __forceinline__ double variance_inv() {
         double s = 0.0;
         for (int p = tid; p < N; p += NT) s += (double)pos[p].z;
         const double mean = block_sum(s) / N;
         double v = 0.0;
-        for (int p = tid; p < N; p += NT) { const double d = (double)pos[p].z - mean; v += d * d; }
+        for (int p = tid; p < N; p += NT) { const double d = __dsub_rn((double)pos[p].z, mean); v = __dadd_rn(v, __dmul_rn(d, d)); }
         const double var = block_sum(v) / N;
         return (var < 0.000001) ? 1000.0 : 0.001 / var;
     }
